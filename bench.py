@@ -375,6 +375,17 @@ def _traffic(kernel):
     return None, None
 
 
+def dump_outputs(out_dir, ids):
+    """Writes the token ids of the windows of the last timed step to out_dir/token_ids.npy: one row per window, padded with
+    -1, float32 (ids below 2^24 are exact).  They are what a caller of the timed path receives, so two builds run with the
+    same arguments can be compared output for output."""
+    rows = np.full((len(ids), max((len(t) for t in ids), default=0)), -1, dtype=np.float32)
+    for i, t in enumerate(ids):
+        rows[i, :len(t)] = t
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "token_ids.npy"), rows)
+
+
 # ----------------------------------------------------------------------------------------------- GPU arm
 def main():
     ap = argparse.ArgumentParser()
@@ -387,12 +398,18 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the logmel / encoder / in-step measurements (profiling runs)")
     ap.add_argument("--e2e-repeats", type=int, default=1)
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs only: do not time the public-API pass")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the token ids of the last step's windows to DIR/token_ids.npy")
     ap.add_argument("--merge", type=int, default=1, help="user batches of 32 windows merged into one device batch (rows are independent)")
     ap.add_argument("--streams", type=int, default=0, help="batches in flight per GPU (shared-weight replicas); default 8 (4 for --config reference)")
     ap.add_argument("--config", default="north_star", choices=["north_star", "reference"],
                     help="north_star: greedy, 4-token prompt (BASELINE configs).  reference: the call shape of /root/reference/transcribe.py:"
                          "107-113 - whisperx defaults (beam_size 5, patience 1, without_timestamps) plus a ~60-token initial_prompt")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     ref_shape = args.config == "reference"
     if not args.streams:
         args.streams = 4 if ref_shape else 8          # beam 5 holds 160 rows of self-K/V per replica (21 GB of workspace each)
@@ -482,15 +499,17 @@ def main():
         return t.tolist()
 
     def throughput_steps(resident, o, l32, l64, steps):
-        """`steps` batches of 32 windows (cycling the full batches of a recording) through the in-flight replicas"""
+        """`steps` batches of 32 windows (cycling the full batches of a recording) through the in-flight replicas
+        -> (ms, audio seconds, launches, clocks, (text, ids) of the last step's windows)"""
         n_full = len(o) // BATCH
 
         def run(first, count):
             idx = np.concatenate([np.arange(((first + i) % n_full) * BATCH, ((first + i) % n_full + 1) * BATCH) for i in range(count)])
-            pipe.run_device_batches(resident, o[idx], l32[idx], BATCH * args.merge)
-            return float(l64[idx].sum()) / 16000.0
+            res = pipe.run_device_batches(resident, o[idx], l32[idx], BATCH * args.merge)
+            return float(l64[idx].sum()) / 16000.0, res
         run(0, args.warmup)
-        return timed(lambda: run(args.warmup, steps))
+        ms, (audio_s, res), launches, clocks = timed(lambda: run(args.warmup, steps))
+        return ms, audio_s, launches, clocks, res[-BATCH:]
 
     line = {"metric": METRIC, "unit": "x real-time", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
             "higher_is_better": True, "vs_baseline": None, "dtype": storage, "data": "synthetic"}
@@ -503,7 +522,9 @@ def main():
         # ------------------------------------------------------------------ N = 1
         resident = pipe.upload(audio_host, offs, lens)        # untimed: `value` is measured with inputs resident in HBM
         warm_replicas(resident, offs, lens32)
-        ms, audio_s, launches, clocks = throughput_steps(resident, offs, lens32, lens, args.steps)
+        ms, audio_s, launches, clocks, last_step = throughput_steps(resident, offs, lens32, lens, args.steps)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, [toks for _, toks in last_step])
         # the whole recording once, resident (the N = 1 point of the strong-scaling curve)
         pipe.run_device_batches(resident, offs, lens32, BATCH)
         ms_hour, _, _, _ = timed(lambda: pipe.run_device_batches(resident, offs, lens32, BATCH))
@@ -586,6 +607,8 @@ def main():
         single = pipe.run_device_batches(full, offs, lens32, BATCH)
         match = [r[1] for r in single] == ids
         del full
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, ids)          # a step here is one pass over the whole recording
     t_e2e = []
     for _ in range(0 if args.skip_e2e else max(1, args.e2e_repeats)):
         barrier()
@@ -602,7 +625,7 @@ def main():
     oo = np.array([int(w["start"] * 16000) for w in own_w], dtype=np.int64)
     ol = np.array([int(w["end"] * 16000) for w in own_w], dtype=np.int64) - oo
     own_res = pipe.upload(own_audio, oo, ol)
-    ms_w, audio_w, _, _ = throughput_steps(own_res, oo, ol.astype(np.int32), ol, args.steps)
+    ms_w, audio_w, _, _, _ = throughput_steps(own_res, oo, ol.astype(np.int32), ol, args.steps)
     ms_w_max = allreduce([ms_w], "max")[0]
     audio_w_sum = allreduce([audio_w], "sum")[0]
     # config 5 at N GPUs: independent replicas, every rank the un-chunked log-mel of its own 1-hour clip (no exchange needed)

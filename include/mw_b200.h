@@ -201,6 +201,39 @@ void mw_decode_gemm_debug(unsigned long long* d_stamps);
 mw_status mw_layernorm(const float* d_x, const float* d_gamma, const float* d_beta, void* d_out_h16,
                        int rows, int d, void* stream);
 
+/* The decode step's own kernels (csrc/decoder.cu) on caller buffers, for tests/test_gpu_decode_step.py.  The launch path is
+ * named by an argument; no A/B environment hook changes what these run.  They may allocate a few bytes and synchronise. */
+enum mw_step_path {
+    MW_STEP_PATH_GREEDY = 0,        /* the step's routing in greedy search: tcgen05 decode GEMM from 96 rows, else mma.sync */
+    MW_STEP_PATH_BEAM = 1,          /* the step's routing of the layer projections in beam search: mma.sync kernels only */
+    MW_STEP_PATH_GREEDY_SOLO = 2,   /* the same two with mw_set_solo on (fused LayerNorm, one-tile K-halved fc2) */
+    MW_STEP_PATH_BEAM_SOLO = 3,
+    MW_STEP_PATH_ROWS16_WT1 = 4,    /* forced kernels: rows16 with one / two 16-row weight tiles per CTA, */
+    MW_STEP_PATH_ROWS16_WT2 = 5,
+    MW_STEP_PATH_KHALF_WT1 = 6,     /* the K-halved kernel (K = 2048 .. 5120) with one / two tiles, */
+    MW_STEP_PATH_KHALF_WT2 = 7,
+    MW_STEP_PATH_GENERIC = 8,       /* the generic kernel (any K % 32 == 0), */
+    MW_STEP_PATH_LN_FUSED = 9,      /* LayerNorm folded into the projection (16-bit output), */
+    MW_STEP_PATH_LN_SEPARATE = 10   /* LayerNorm, then the projection (beam routing), as two launches */
+};
+/* out[R,N] = X[R,K] . W[N,K]^T (+bias[N]) (flags&1: GELU) (+resid f32 [R,N]); out h16, or f32 when flags&2.  With gamma and
+ * beta, X = LayerNorm(x_f32 [R,K]) and x_h16 is the scratch the stand-alone LayerNorm writes; otherwise X = x_h16.  A forced
+ * kernel that does not exist for K returns MW_ERR_UNSUPPORTED. */
+mw_status mw_step_projection_h16(const void* d_x_h16, const float* d_x_f32, const float* d_gamma, const float* d_beta,
+                                 const void* d_w, const float* d_bias, const float* d_resid, void* d_out, int R, int N, int K,
+                                 int flags, int path, void* stream);
+/* Self-attention of one step: appends k, v of qkv h16 [R, 3d] at position pos of the caches h16 [R, ctx, d], then attends over
+ * pos + 1 keys; key j < pos of row r is read from cache row d_idx[r*ctx + j] (int32 [R, ctx]; NULL = row r).  out h16 [R, d]. */
+mw_status mw_step_self_attention_h16(const void* d_qkv, void* d_k_cache, void* d_v_cache, const int32_t* d_idx, int R,
+                                     int n_heads, int ctx, int pos, void* d_out, void* stream);
+/* Causal self-attention of the batched prompt prefill: qkv h16 [B*P, 3d], row b*P + p sees keys 0..p of its sequence. */
+mw_status mw_step_prefill_attention_h16(const void* d_qkv, int B, int P, int n_heads, void* d_out, void* stream);
+/* Cross-attention: G queries per sequence q h16 [B*G, d] over the sequence's keys/values kv h16 [B*T, 2d] (k | v);
+ * out h16 [B*G, d].  G = 1: the streaming kernel with unr = 4 or 8 loads in flight per lane; G = 2..8: the grouped kernel of
+ * beam search (G*T*4 bytes of scores must fit 96 KB). */
+mw_status mw_step_cross_attention_h16(const void* d_q, const void* d_kv, int B, int G, int T, int n_heads, int unr,
+                                      void* d_out, void* stream);
+
 /* VAD front end (SURVEY.md §8f rank 1): RMS of consecutive frames of `frame` samples, d_out float32 [n / frame].
  * Feeds the energy VAD so the waveform is uploaded once and never revisited by the host. */
 mw_status mw_frame_rms(const float* d_audio, int64_t n, int frame, float* d_out, void* stream);

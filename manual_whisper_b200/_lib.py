@@ -82,6 +82,13 @@ SIGNATURES = {
     "mw_vad_windows": (C.c_int32, [C.c_void_p, C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double,
                                    C.c_double, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "mw_layernorm": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "mw_step_projection_h16": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "mw_step_self_attention_h16": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                               C.c_void_p, C.c_void_p]),
+    "mw_step_prefill_attention_h16": (C.c_int32, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "mw_step_cross_attention_h16": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                                C.c_void_p]),
     "mw_w2v_create": (C.c_int32, [C.POINTER(W2vConfigC), C.POINTER(WeightTableC), C.POINTER(C.c_void_p)]),
     "mw_w2v_destroy": (None, [C.c_void_p]),
     "mw_w2v_workspace_bytes": (C.c_int64, [C.c_void_p]),

@@ -494,16 +494,68 @@ skinny_gemm_rows32_khalf_kernel(const mw_h* __restrict__ X, int ldx, const mw_h*
     }
 }
 
+// Which kernel a decode-step projection runs.  SK_STEP is the step's own routing, A/B hooks included (read once per process);
+// SK_ROUTE is the same routing with every hook at its default; the others force one kernel (mw_step_projection_h16).
+enum SkPath { SK_STEP, SK_ROUTE, SK_ROWS16_WT1, SK_ROWS16_WT2, SK_KHALF_WT1, SK_KHALF_WT2, SK_GENERIC, SK_LN_FUSED, SK_LN_SEPARATE };
+
+struct SkHooks {
+    bool one_tile;      // MW_SKINNY_WT=1: one weight tile per CTA in the mma.sync projections
+    bool no_khalf;      // MW_SKINNY_KHALF=0: no K-halved kernel
+    int khalf_wt;       // MW_KHALF_WT: 0 = by mw_set_solo, 1 / 2 = forced
+    int dg_min_rows;    // MW_DG_MIN_ROWS: rows from which the tcgen05 decode GEMM takes over
+    int ln_fuse;        // MW_LN_FUSE: -1 = by mw_set_solo, 0 never, 1 always
+    bool prefetch;      // MW_PREFETCH=0 switches the L2 prefetch of the next projection's weights off
+};
+constexpr SkHooks SK_DEFAULT_HOOKS = {false, false, 0, 96, -1, true};
+const SkHooks& sk_env_hooks() {
+    static const SkHooks h = [] {
+        SkHooks v = SK_DEFAULT_HOOKS;
+        const char* e;
+        if ((e = getenv("MW_SKINNY_WT"))) v.one_tile = e[0] == '1';
+        if ((e = getenv("MW_SKINNY_KHALF"))) v.no_khalf = e[0] == '0';
+        if ((e = getenv("MW_KHALF_WT"))) v.khalf_wt = atoi(e);
+        if ((e = getenv("MW_DG_MIN_ROWS"))) v.dg_min_rows = atoi(e);
+        if ((e = getenv("MW_LN_FUSE"))) v.ln_fuse = atoi(e);
+        if ((e = getenv("MW_PREFETCH"))) v.prefetch = e[0] != '0';
+        return v;
+    }();
+    return h;
+}
+const SkHooks& sk_hooks(SkPath path) { return path == SK_STEP ? sk_env_hooks() : SK_DEFAULT_HOOKS; }
+
+// The tuned projections of skinny_gemm (its MW_SK table): warps per CTA for K = KB * NW * 32, 0 when K has no entry.
+// The K-halved kernel serves the 16-warp entries; two weight tiles fit the registers for KB <= 5 with at most 8 warps.
+int sk_table_warps(int K) {
+    switch (K) {
+        case 128: case 384: return 4;
+        case 256: case 512: case 768: case 1024: case 1280: case 1536: return 8;
+        case 2048: case 3072: case 4096: case 5120: return 16;
+        default: return 0;
+    }
+}
+bool sk_has_rows16_wt2(int K) { const int nw = sk_table_warps(K); return nw && nw <= 8 && K / (nw * 32) <= 5; }
+bool sk_has_khalf(int K) { const int nw = sk_table_warps(K); return nw == 16 && (K / (nw * 32)) % 2 == 0 && K / (nw * 32) / 2 <= 5; }
+bool sk_has_ln_fused(int K) { return sk_has_rows16_wt2(K); }    // the MW_SKLN table of skinny_gemm_ln
+
 template <int KB, int NW>
 mw_status launch_rows16(const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
-                        int ldo, int R, int N, int K, int flags, cudaStream_t st, const char* pf, int pf_lines, bool solo) {
+                        int ldo, int R, int N, int K, int flags, cudaStream_t st, const char* pf, int pf_lines, bool solo,
+                        SkPath path) {
     constexpr int WT = (NW <= 8 && KB <= 5) ? 2 : 1;          // two weight tiles where the registers allow it
-    static const bool one_tile = [] { const char* e = getenv("MW_SKINNY_WT"); return e && e[0] == '1'; }();   // A/B hook
+    const SkHooks& hk = sk_hooks(path);
+    const bool routed = path == SK_STEP || path == SK_ROUTE;
+    if ((path == SK_KHALF_WT1 || path == SK_KHALF_WT2) && !(NW == 16 && KB % 2 == 0 && KB / 2 <= 5)) {
+        set_error("skinny gemm: no K-halved kernel for K=%d", K);
+        return MW_ERR_UNSUPPORTED;
+    }
+    if (path == SK_ROWS16_WT2 && WT != 2) {
+        set_error("skinny gemm: no two-tile rows16 kernel for K=%d", K);
+        return MW_ERR_UNSUPPORTED;
+    }
     if constexpr (NW == 16 && KB % 2 == 0 && KB / 2 <= 5) {
-        static const bool no_khalf = [] { const char* e = getenv("MW_SKINNY_KHALF"); return e && e[0] == '0'; }();
-        if (!one_tile && !no_khalf) {
-            static const int khalf_wt = [] { const char* e = getenv("MW_KHALF_WT"); return e ? atoi(e) : 0; }();   // A/B hook
-            if (khalf_wt == 1 || (khalf_wt == 0 && solo)) {       // a lone batch: 3.87 -> 3.76 ms per single-stream step
+        if ((routed && !hk.one_tile && !hk.no_khalf) || path == SK_KHALF_WT1 || path == SK_KHALF_WT2) {
+            const bool one = routed ? (hk.khalf_wt == 1 || (hk.khalf_wt == 0 && solo)) : path == SK_KHALF_WT1;
+            if (one) {       // a lone batch: 3.87 -> 3.76 ms per single-stream step
                 dim3 grid(ceil_div(N, 16), ceil_div(R, 32));
                 launch_chained(skinny_gemm_rows32_khalf_kernel<KB / 2, NW, 1>, grid, dim3(NW * 32), 0, st, (const mw_h*)X, ldx,
                                (const mw_h*)W, ldw, bias, resid, out, ldo, R, N, K, flags, pf, pf_lines);
@@ -516,7 +568,7 @@ mw_status launch_rows16(const void* X, int ldx, const void* W, int ldw, const fl
             return MW_OK;
         }
     }
-    if (WT == 2 && !one_tile) {
+    if (WT == 2 && ((routed && !hk.one_tile) || path == SK_ROWS16_WT2)) {
         dim3 grid(ceil_div(N, 32), ceil_div(R, 32));
         launch_chained(skinny_gemm_rows16_kernel<KB, NW, WT>, grid, dim3(NW * 32), 0, st, (const mw_h*)X, ldx, (const mw_h*)W, ldw,
                        bias, resid, out, ldo, R, N, K, flags, pf, pf_lines);
@@ -532,18 +584,24 @@ mw_status launch_rows16(const void* X, int ldx, const void* W, int ldw, const fl
 // `next_w` / `next_bytes`: the weight matrix of the projection that follows this one in the step (prefetched into L2)
 mw_status skinny_gemm(const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
                       int ldo, int R, int N, int K, int flags, cudaStream_t st, bool allow_dg = true,
-                      const void* next_w = nullptr, int64_t next_bytes = 0, bool solo = false) {
-    static const bool prefetch_on = [] { const char* e = getenv("MW_PREFETCH"); return !(e && e[0] == '0'); }();   // A/B hook
-    const char* pf = prefetch_on ? (const char*)next_w : nullptr;
+                      const void* next_w = nullptr, int64_t next_bytes = 0, bool solo = false, SkPath path = SK_STEP) {
+    const SkHooks& hk = sk_hooks(path);
+    const bool routed = path == SK_STEP || path == SK_ROUTE;
+    const char* pf = hk.prefetch ? (const char*)next_w : nullptr;
     const int pf_lines = pf ? (int)(next_bytes / 128) : 0;
     // R >= MW_DG_MIN_ROWS rows (merged greedy batches): the weight-stationary tcgen05 kernel (decode_gemm.cu) streams W once
     // for all rows; the mma.sync kernels below re-read it per 32-row block (from L2 after the first block) and stay in charge
     // of the 32-row batches they were tuned on and of beam search, where they measured faster (DESIGN.md section 4: a decode
     // step is a chain of ~360 latency-bound launches, so bytes saved do not buy time unless the launch is also shorter).
-    static const int dg_min_rows = [] { const char* e = getenv("MW_DG_MIN_ROWS"); return e ? atoi(e) : 96; }();
-    if (allow_dg && R >= dg_min_rows && decode_gemm_supported(ldx, ldw, R, N, K))
-        return decode_gemm_launch(X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st);
-#define MW_SK(kb, nw) if (K == kb * nw * 32) return launch_rows16<kb, nw>(X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st, pf, pf_lines, solo)
+    // The step passes allow_dg = (beam <= 1) for the layer projections; the vocabulary projection (enqueue_logits) keeps the
+    // default, so at R >= 96 rows it runs on the decode GEMM in beam search as well.
+    if (routed && allow_dg && R >= hk.dg_min_rows && decode_gemm_supported(ldx, ldw, R, N, K))
+        return decode_gemm_launch(X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st, path == SK_STEP);
+    if (!routed && path != SK_GENERIC && !sk_table_warps(K)) {
+        set_error("skinny gemm: no tuned kernel for K=%d (the generic kernel serves it)", K);
+        return MW_ERR_UNSUPPORTED;
+    }
+#define MW_SK(kb, nw) if (path != SK_GENERIC && K == kb * nw * 32) return launch_rows16<kb, nw>(X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st, pf, pf_lines, solo, path)
     MW_SK(5, 8);    // 1280  (large)
     MW_SK(10, 16);  // 5120  (large ffn)
     MW_SK(4, 8);    // 1024  (medium)
@@ -586,14 +644,16 @@ __global__ void embed_kernel(const int* __restrict__ cur_tok, const mw_h* __rest
 // 16-bit operand twice in the plain kernels costs nothing at eight streams.)
 mw_status skinny_gemm_ln(const float* x, const float* gamma, const float* beta, void* ln_buf, const void* W, const float* bias,
                          void* out, int ldo, int R, int N, int K, int flags, cudaStream_t st, bool allow_dg, const void* next_w,
-                         int64_t next_bytes, bool solo) {
-    static const int fuse_env = [] { const char* e = getenv("MW_LN_FUSE"); return e ? atoi(e) : -1; }();   // A/B hook: 0 never, 1 always
-    const bool fuse = fuse_env < 0 ? solo : fuse_env != 0;
-    static const bool prefetch_on = [] { const char* e = getenv("MW_PREFETCH"); return !(e && e[0] == '0'); }();
-    static const int dg_min_rows = [] { const char* e = getenv("MW_DG_MIN_ROWS"); return e ? atoi(e) : 96; }();
-    const bool to_dg = allow_dg && R >= dg_min_rows && decode_gemm_supported(K, K, R, N, K);
+                         int64_t next_bytes, bool solo, SkPath path = SK_STEP) {
+    const SkHooks& hk = sk_hooks(path);
+    const bool fuse = path == SK_LN_FUSED || ((path == SK_STEP || path == SK_ROUTE) && (hk.ln_fuse < 0 ? solo : hk.ln_fuse != 0));
+    const bool to_dg = path != SK_LN_FUSED && allow_dg && R >= hk.dg_min_rows && decode_gemm_supported(K, K, R, N, K);
+    if (path == SK_LN_FUSED && (!sk_has_ln_fused(K) || (flags & SK_FLAG_F32))) {
+        set_error("skinny gemm: no fused LayerNorm projection for K=%d%s", K, (flags & SK_FLAG_F32) ? " with fp32 output" : "");
+        return MW_ERR_UNSUPPORTED;
+    }
     if (fuse && !to_dg && !(flags & SK_FLAG_F32)) {
-        const char* pf = prefetch_on ? (const char*)next_w : nullptr;
+        const char* pf = hk.prefetch ? (const char*)next_w : nullptr;
         const int pf_lines = pf ? (int)(next_bytes / 128) : 0;
 #define MW_SKLN(kb, nw) if (K == kb * nw * 32) return launch_ln_rows16<kb, nw>(x, gamma, beta, W, K, bias, out, ldo, R, N, flags, st, pf, pf_lines)
         MW_SKLN(5, 8);    // 1280  (large)
@@ -607,7 +667,8 @@ mw_status skinny_gemm_ln(const float* x, const float* gamma, const float* beta, 
     }
     mw_status r = layernorm_launch(x, gamma, beta, ln_buf, R, K, st);
     if (r != MW_OK) return r;
-    return skinny_gemm(ln_buf, K, W, K, bias, nullptr, out, ldo, R, N, K, flags, st, allow_dg, next_w, next_bytes);
+    return skinny_gemm(ln_buf, K, W, K, bias, nullptr, out, ldo, R, N, K, flags, st, allow_dg, next_w, next_bytes, false,
+                       path == SK_STEP ? SK_STEP : SK_ROUTE);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1007,9 +1068,9 @@ template <int G>
 mw_status launch_cross_grouped(const mw_h* q, int ldq, const mw_h* k, const mw_h* v, int64_t key_stride,
                                int n_keys, mw_h* out, int ldo, int n_heads, int B, cudaStream_t st) {
     const size_t smem = (size_t)G * n_keys * sizeof(float);
+    MW_REQUIRE(smem <= 96 * 1024, "cross attention: %zu bytes of scores exceed shared memory", smem);
     static PerDeviceOnce attr_once;
     MW_CUDA_CHECK(attr_once.run([&] { return cudaFuncSetAttribute(cross_attn_grouped_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); }));
-    MW_REQUIRE(smem <= 96 * 1024, "cross attention: %zu bytes of scores exceed shared memory", smem);
     launch_chained(cross_attn_grouped_kernel<G>, dim3(n_heads, B), dim3(128), smem, st, q, ldq, k, v, key_stride, n_keys, out, ldo);
     MW_LAUNCH_CHECK();
     return MW_OK;
@@ -2158,4 +2219,122 @@ extern "C" mw_status mw_set_solo(mw_model* m, int solo) {
 extern "C" void mw_debug_step_parts(int parts) {
     mw::g_step_parts.store(parts);
     mw::g_step_parts_epoch.fetch_add(1);
+}
+
+// ---- test entry points (include/mw_b200.h): the decode step's kernels on caller buffers, the launch path named by an argument.
+// No A/B hook changes what they run.  Shapes and the path are checked before any pointer, and all of it before anything is
+// launched, so a rejected call touches no memory.
+extern "C" mw_status mw_step_projection_h16(const void* d_x_h16, const float* d_x_f32, const float* d_gamma, const float* d_beta,
+                                            const void* d_w, const float* d_bias, const float* d_resid, void* d_out, int R, int N,
+                                            int K, int flags, int path, void* stream) {
+    MW_REQUIRE(R >= 1 && R <= 65535 * 32 && N >= 1 && K >= 32 && K % 32 == 0,
+               "mw_step_projection_h16: R=%d N=%d K=%d (K a multiple of 32)", R, N, K);
+    MW_REQUIRE(flags >= 0 && flags <= 3, "mw_step_projection_h16: flags=%d (1 = GELU, 2 = fp32 out)", flags);
+    MW_REQUIRE(path >= MW_STEP_PATH_GREEDY && path <= MW_STEP_PATH_LN_SEPARATE, "mw_step_projection_h16: unknown path %d", path);
+    const bool ln = d_gamma || d_beta;
+    const bool ln_path = path == MW_STEP_PATH_LN_FUSED || path == MW_STEP_PATH_LN_SEPARATE;
+    const bool forced = path >= MW_STEP_PATH_ROWS16_WT1 && !ln_path;
+    MW_REQUIRE(ln || !ln_path, "mw_step_projection_h16: path %d is a LayerNorm path: gamma and beta are required", path);
+    MW_REQUIRE(!ln || !forced, "mw_step_projection_h16: path %d forces one projection kernel on x_h16: no LayerNorm", path);
+    MW_REQUIRE(!ln || !d_resid, "mw_step_projection_h16: a LayerNorm projection takes no residual");
+    MW_REQUIRE(!ln || (K % 128 == 0 && K <= 2048), "mw_step_projection_h16: LayerNorm over K=%d (a multiple of 128 up to 2048)", K);
+    const char* missing = nullptr;
+    switch (path) {
+        case MW_STEP_PATH_ROWS16_WT1: if (!sk_table_warps(K)) missing = "rows16"; break;
+        case MW_STEP_PATH_ROWS16_WT2: if (!sk_has_rows16_wt2(K)) missing = "two-tile rows16"; break;
+        case MW_STEP_PATH_KHALF_WT1: case MW_STEP_PATH_KHALF_WT2: if (!sk_has_khalf(K)) missing = "K-halved"; break;
+        case MW_STEP_PATH_LN_FUSED: if (!sk_has_ln_fused(K) || (flags & SK_FLAG_F32)) missing = "fused LayerNorm (16-bit output)"; break;
+        default: break;
+    }
+    if (missing) {
+        set_error("mw_step_projection_h16: no %s kernel for K=%d", missing, K);
+        return MW_ERR_UNSUPPORTED;
+    }
+    MW_REQUIRE(d_x_h16 && d_w && d_out && (!ln || (d_x_f32 && d_gamma && d_beta)), "mw_step_projection_h16: null pointer");
+    MW_REQUIRE((uintptr_t)d_x_h16 % 16 == 0 && (uintptr_t)d_w % 16 == 0 && (uintptr_t)d_x_f32 % 16 == 0,
+               "mw_step_projection_h16: x and W must be 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    SkPath p = SK_ROUTE;
+    bool allow_dg = false, solo = false;
+    switch (path) {
+        case MW_STEP_PATH_GREEDY: allow_dg = true; break;
+        case MW_STEP_PATH_GREEDY_SOLO: allow_dg = true; solo = true; break;
+        case MW_STEP_PATH_BEAM_SOLO: solo = true; break;
+        case MW_STEP_PATH_ROWS16_WT1: p = SK_ROWS16_WT1; break;
+        case MW_STEP_PATH_ROWS16_WT2: p = SK_ROWS16_WT2; break;
+        case MW_STEP_PATH_KHALF_WT1: p = SK_KHALF_WT1; break;
+        case MW_STEP_PATH_KHALF_WT2: p = SK_KHALF_WT2; break;
+        case MW_STEP_PATH_GENERIC: p = SK_GENERIC; break;
+        case MW_STEP_PATH_LN_FUSED: p = SK_LN_FUSED; break;
+        case MW_STEP_PATH_LN_SEPARATE: p = SK_LN_SEPARATE; break;
+        default: break;
+    }
+    if (ln)
+        return skinny_gemm_ln(d_x_f32, d_gamma, d_beta, const_cast<void*>(d_x_h16), d_w, d_bias, d_out, N, R, N, K, flags, st,
+                              allow_dg, nullptr, 0, solo, p);
+    return skinny_gemm(d_x_h16, K, d_w, K, d_bias, d_resid, d_out, N, R, N, K, flags, st, allow_dg, nullptr, 0, solo, p);
+}
+
+extern "C" mw_status mw_step_self_attention_h16(const void* d_qkv, void* d_k_cache, void* d_v_cache, const int32_t* d_idx, int R,
+                                                int n_heads, int ctx, int pos, void* d_out, void* stream) {
+    MW_REQUIRE(R >= 1 && R <= 65535 && n_heads >= 1 && n_heads <= 65535 && ctx >= 1 && ctx <= 12 * 1024 && pos >= 0 && pos < ctx,
+               "mw_step_self_attention_h16: R=%d n_heads=%d ctx=%d pos=%d", R, n_heads, ctx, pos);
+    MW_REQUIRE(d_qkv && d_k_cache && d_v_cache && d_out, "mw_step_self_attention_h16: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int d = n_heads * 64;
+    const mw_h* qkv = (const mw_h*)d_qkv;
+    DecCtl h_ctl = {pos, 0, 0, 0};
+    DecCtl* ctl = nullptr;
+    MW_CUDA_CHECK(cudaMalloc((void**)&ctl, sizeof(DecCtl)));
+    cudaError_t e = cudaMemcpyAsync(ctl, &h_ctl, sizeof(DecCtl), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess)
+        e = launch_chained(decode_attn_kernel<true>, dim3(n_heads, R), dim3(128), ctx * sizeof(float), st, qkv, 3 * d,
+                           (mw_h*)d_k_cache, (mw_h*)d_v_cache, (int64_t)d, (int64_t)ctx, (const int*)d_idx, ctx, (const DecCtl*)ctl, 0,
+                           1, qkv + d, qkv + 2 * d, 3 * d, (mw_h*)d_out, d, 0);
+    if (e == cudaSuccess) { count_launch(); e = cudaStreamSynchronize(st); }      // h_ctl is read by the copy until then
+    cudaFree(ctl);
+    if (e != cudaSuccess) { set_error("mw_step_self_attention_h16: %s", cudaGetErrorString(e)); return MW_ERR_CUDA; }
+    return MW_OK;
+}
+
+extern "C" mw_status mw_step_prefill_attention_h16(const void* d_qkv, int B, int P, int n_heads, void* d_out, void* stream) {
+    MW_REQUIRE(B >= 1 && P >= 1 && P <= 16 * 1024 && (int64_t)B * P <= 65535 && n_heads >= 1,
+               "mw_step_prefill_attention_h16: B=%d P=%d n_heads=%d", B, P, n_heads);
+    MW_REQUIRE(d_qkv && d_out, "mw_step_prefill_attention_h16: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    static PerDeviceOnce attr_once;
+    MW_CUDA_CHECK(attr_once.run([] { return cudaFuncSetAttribute(decode_attn_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024); }));
+    const int d = n_heads * 64;
+    mw_h* qkv = (mw_h*)const_cast<void*>(d_qkv);       // read only: the kernel writes the cache only when SELF
+    decode_attn_kernel<false><<<dim3(n_heads, B * P), 128, P * sizeof(float), st>>>(qkv, 3 * d, qkv + d, qkv + 2 * d, 3 * d, P, nullptr,
+                                                                                   0, nullptr, P, P, nullptr, nullptr, 0, (mw_h*)d_out, d, P);
+    MW_LAUNCH_CHECK();
+    return MW_OK;
+}
+
+extern "C" mw_status mw_step_cross_attention_h16(const void* d_q, const void* d_kv, int B, int G, int T, int n_heads, int unr,
+                                                 void* d_out, void* stream) {
+    MW_REQUIRE(B >= 1 && B <= 65535 && T >= 1 && n_heads >= 1 && n_heads <= 65535,
+               "mw_step_cross_attention_h16: B=%d T=%d n_heads=%d", B, T, n_heads);
+    MW_REQUIRE(G >= 1 && G <= MAX_BEAM, "mw_step_cross_attention_h16: G=%d outside 1..%d", G, MAX_BEAM);
+    MW_REQUIRE(G > 1 || unr == 4 || unr == 8, "mw_step_cross_attention_h16: unr=%d (4 or 8)", unr);
+    MW_REQUIRE(d_q && d_kv && d_out, "mw_step_cross_attention_h16: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int d = n_heads * 64;
+    const mw_h* q = (const mw_h*)d_q;
+    const mw_h* kv = (const mw_h*)d_kv;
+    mw_h* out = (mw_h*)d_out;
+    if (G == 1) {
+        if (unr == 8)
+            launch_chained(cross_attn_stream_kernel<8>, dim3(n_heads, B), dim3(128), 0, st, q, d, kv, kv + d, (int64_t)(2 * d), T, out, d,
+                           (const char*)nullptr, 0);
+        else
+            launch_chained(cross_attn_stream_kernel<4>, dim3(n_heads, B), dim3(128), 0, st, q, d, kv, kv + d, (int64_t)(2 * d), T, out, d,
+                           (const char*)nullptr, 0);
+        MW_LAUNCH_CHECK();
+        return MW_OK;
+    }
+#define MW_XG(g) case g: return launch_cross_grouped<g>(q, d, kv, kv + d, 2 * d, T, out, d, n_heads, B, st)
+    switch (G) { MW_XG(2); MW_XG(3); MW_XG(4); MW_XG(5); MW_XG(6); MW_XG(7); default: MW_XG(8); }
+#undef MW_XG
 }

@@ -50,6 +50,40 @@ def test_argument_errors_do_not_need_a_gpu(built_lib):
     assert lib.mw_logmel(None, None, 0, None, None, 1, None, None, None) == 1
 
 
+def test_step_entry_points_reject_bad_arguments_without_a_gpu(built_lib):
+    """Shapes, paths and pointers are checked before anything touches the device; every call here is rejected up front."""
+    from manual_whisper_b200 import _lib
+    lib = _lib.load()
+    proj = lib.mw_step_projection_h16
+    # forced kernels that do not exist for K (checked before the pointers, which are null here)
+    # (gamma and beta only mark the LayerNorm path: x, W and out are null, so nothing could be launched)
+    for path, K in [(4, 640), (5, 1536), (5, 2048), (6, 1280), (7, 640), (7, 2560), (9, 1536), (9, 2048)]:
+        g = 16 if path == 9 else None
+        assert proj(None, None, g, g, None, None, None, None, 32, 64, K, 0, path, None) == 3, (path, K)
+        assert b"no " in lib.mw_last_error() and str(K).encode() in lib.mw_last_error()
+    assert proj(None, None, 16, 16, None, None, None, None, 32, 64, 512, 2, 9, None) == 3    # fused LN has no fp32 output
+    # bad shapes, flags and paths
+    assert proj(None, None, None, None, None, None, None, None, 32, 64, 100, 0, 0, None) == 1
+    assert proj(None, None, None, None, None, None, None, None, 0, 64, 128, 0, 0, None) == 1
+    assert proj(None, None, None, None, None, None, None, None, 32, 64, 128, 4, 0, None) == 1
+    assert proj(None, None, None, None, None, None, None, None, 32, 64, 128, 0, 11, None) == 1
+    assert proj(None, None, None, None, None, None, None, None, 32, 64, 128, 0, 10, None) == 1    # LN path without gamma
+    # supported shapes with null pointers
+    for path in range(9):
+        K = 2048 if path in (6, 7) else 512
+        assert proj(None, None, None, None, None, None, None, None, 32, 64, K, 0, path, None) == 1
+        assert b"null" in lib.mw_last_error()
+    assert lib.mw_step_self_attention_h16(None, None, None, None, 4, 6, 448, 0, None, None) == 1
+    assert b"null" in lib.mw_last_error()
+    assert lib.mw_step_self_attention_h16(None, None, None, None, 4, 6, 448, 448, None, None) == 1     # pos outside ctx
+    assert lib.mw_step_prefill_attention_h16(None, 2, 16, 6, None, None) == 1
+    cross = lib.mw_step_cross_attention_h16
+    assert cross(None, None, 2, 9, 1500, 6, 4, None, None) == 1 and b"G=9" in lib.mw_last_error()
+    assert cross(None, None, 2, 0, 1500, 6, 4, None, None) == 1
+    assert cross(None, None, 2, 1, 1500, 6, 2, None, None) == 1 and b"unr" in lib.mw_last_error()
+    assert cross(None, None, 2, 1, 1500, 6, 8, None, None) == 1 and b"null" in lib.mw_last_error()
+
+
 def test_sass_is_blackwell_native(built_lib):
     """tcgen05.mma -> UTCHMMA, tcgen05.ld -> LDTM, TMA -> UTMALDG must be present in the sm_100a SASS."""
     sass = subprocess.check_output(["cuobjdump", "-sass", str(built_lib)], text=True)

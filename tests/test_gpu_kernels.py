@@ -105,7 +105,8 @@ def test_encoder_attention(lib, B, T, H):
     assert (out.float() - ref).abs().max().item() < 2 ** -7 * ref.abs().max().item() + 2e-3
 
 
-@pytest.mark.parametrize("rows,d", [(1, 128), (1000, 384), (37, 1280), (48000, 1280)])
+@pytest.mark.parametrize("rows,d", [(1, 128), (1000, 384), (37, 1280), (48000, 1280),
+                                    (33, 512), (33, 640), (33, 1536), (33, 2048)])    # the MAXV boundaries of layernorm_launch
 def test_layernorm(lib, rows, d):
     from manual_whisper_b200 import _lib
     dev = torch.device("cuda:0")

@@ -200,6 +200,25 @@ void mw_debug_step_parts(int parts);
 void mw_decode_gemm_debug(unsigned long long* d_stamps);
 mw_status mw_layernorm(const float* d_x, const float* d_gamma, const float* d_beta, void* d_out_h16,
                        int rows, int d, void* stream);
+/* The tcgen05 GEMM in the full geometry of struct GemmArgs (csrc/gemm.cuh), for tests/test_gpu_tensor_core_paths.py:
+ * out[b*out_batch_rows + out_row_off + m, n] (ld_out) = sum_k A[b*a_batch_stride + m*a_row_stride + k] W[n*w_row_stride + k]
+ *     (+bias[n]) (gelu) (+resid[(b*res_batch_rows + m)*ld_res + n]).
+ * A rows may overlap (a_row_stride < K); resid may equal out.  Shapes and strides are checked before any pointer. */
+mw_status mw_gemm_general_h16(const void* d_a, int64_t a_row_stride, int64_t a_batch_stride, const void* d_w, int64_t w_row_stride,
+                              const float* d_bias, const float* d_resid, int64_t res_batch_rows, int64_t ld_res,
+                              void* d_out, int64_t out_batch_rows, int64_t out_row_off, int64_t ld_out,
+                              int batch, int M, int N, int K, int gelu, int out_f32, void* stream);
+/* attention_launch_general: q [B, Tq, ldq] head h at column colq0 + 64h; k|v [B, Tk, ldkv] at colk0 / colv0 + 64h;
+ * out [B*Tq, out_ld] head h at column 64h; d_kv_lens (may be NULL, only with Tq == Tk): keys >= len masked, wholly padded
+ * query tiles untouched (the ragged contract of attention_launch, csrc/kernels.cuh).  Column ranges are checked before any
+ * pointer. */
+mw_status mw_attention_general_h16(const void* d_q, int64_t ldq, int colq0, const void* d_kv, int64_t ldkv, int colk0, int colv0,
+                                   void* d_out, int out_ld, int B, int Tq, int Tk, int n_heads, const int32_t* d_kv_lens,
+                                   void* stream);
+/* LayerNorm variants: mode 1 = GELU(LN) -> h16, 2 = GELU(LN) -> f32 (d <= 512); 3 = LN -> h16 AND written back over x in f32.
+ * Mode 0 is mw_layernorm.  Shape and mode are checked before any pointer. */
+mw_status mw_layernorm_mode(float* d_x, const float* d_gamma, const float* d_beta, void* d_out, int rows, int d, int mode,
+                            void* stream);
 
 /* The decode step's own kernels (csrc/decoder.cu) on caller buffers, for tests/test_gpu_decode_step.py.  The launch path is
  * named by an argument; no A/B environment hook changes what these run.  They may allocate a few bytes and synchronise. */

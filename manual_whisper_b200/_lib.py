@@ -82,6 +82,12 @@ SIGNATURES = {
     "mw_vad_windows": (C.c_int32, [C.c_void_p, C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double,
                                    C.c_double, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "mw_layernorm": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "mw_gemm_general_h16": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
+                                        C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int,
+                                        C.c_int, C.c_int, C.c_void_p]),
+    "mw_attention_general_h16": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p,
+                                             C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "mw_layernorm_mode": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "mw_step_projection_h16": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                            C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "mw_step_self_attention_h16": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,

@@ -299,3 +299,21 @@ mw_status attention_launch(const void* d_qkv, void* d_out, int B, int T, int n_h
 extern "C" mw_status mw_attention_h16(const void* d_qkv, void* d_out, int B, int T, int n_heads, void* stream) {
     return mw::attention_launch(d_qkv, d_out, B, T, n_heads, (cudaStream_t)stream, nullptr);
 }
+
+extern "C" mw_status mw_attention_general_h16(const void* d_q, int64_t ldq, int colq0, const void* d_kv, int64_t ldkv, int colk0,
+                                               int colv0, void* d_out, int out_ld, int B, int Tq, int Tk, int n_heads,
+                                               const int32_t* d_kv_lens, void* stream) {
+    // shapes and column ranges first, then the pointers: a rejected call touches no memory
+    MW_REQUIRE(B > 0 && Tq > 0 && Tk > 0 && n_heads > 0, "mw_attention_general_h16: bad shape B=%d Tq=%d Tk=%d n_heads=%d",
+               B, Tq, Tk, n_heads);
+    const int64_t w = (int64_t)mw::DH * n_heads;
+    MW_REQUIRE(ldq % 8 == 0 && ldkv % 8 == 0 && out_ld % 8 == 0 && colq0 % 8 == 0 && colk0 % 8 == 0 && colv0 % 8 == 0,
+               "mw_attention_general_h16: leading dimensions and column offsets must be multiples of 8");
+    MW_REQUIRE(colq0 >= 0 && colq0 + w <= ldq && colk0 >= 0 && colk0 + w <= ldkv && colv0 >= 0 && colv0 + w <= ldkv && w <= out_ld,
+               "mw_attention_general_h16: %d heads do not fit: colq0=%d ldq=%lld colk0=%d colv0=%d ldkv=%lld out_ld=%d", n_heads,
+               colq0, (long long)ldq, colk0, colv0, (long long)ldkv, out_ld);
+    MW_REQUIRE(!d_kv_lens || Tq == Tk, "mw_attention_general_h16: kv_lens needs Tq == Tk (Tq=%d Tk=%d)", Tq, Tk);
+    MW_REQUIRE(d_q && d_kv && d_out, "mw_attention_general_h16: null pointer");
+    return mw::attention_launch_general(d_q, ldq, colq0, d_kv, ldkv, colk0, colv0, d_out, out_ld, B, Tq, Tk, n_heads,
+                                        (cudaStream_t)stream, d_kv_lens);
+}

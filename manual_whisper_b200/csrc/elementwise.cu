@@ -167,6 +167,20 @@ extern "C" mw_status mw_layernorm(const float* d_x, const float* d_gamma, const 
     return mw::layernorm_launch(d_x, d_gamma, d_beta, d_out_bf16, rows, d, (cudaStream_t)stream);
 }
 
+extern "C" mw_status mw_layernorm_mode(float* d_x, const float* d_gamma, const float* d_beta, void* d_out, int rows, int d, int mode,
+                                       void* stream) {
+    // shape and mode first, then the pointers: a rejected call touches no memory
+    MW_REQUIRE(mode >= 0 && mode <= 3, "mw_layernorm_mode: mode=%d must be 0..3", mode);
+    const int max_d = (mode == 1 || mode == 2) ? 512 : 2048;
+    MW_REQUIRE(rows >= 0 && d % 128 == 0 && d >= 128 && d <= max_d,
+               "mw_layernorm_mode: rows=%d d=%d (mode %d needs d %% 128 == 0 in [128, %d])", rows, d, mode, max_d);
+    MW_REQUIRE(d_x && d_gamma && d_beta && d_out, "mw_layernorm_mode: null pointer");
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (mode == 0) return mw::layernorm_launch(d_x, d_gamma, d_beta, d_out, rows, d, st);
+    if (mode == 3) return mw::layernorm_dual_launch(d_x, d_gamma, d_beta, d_out, rows, d, st);
+    return mw::layernorm_act_launch(d_x, d_gamma, d_beta, d_out, rows, d, mode, st);
+}
+
 extern "C" mw_status mw_frame_rms(const float* d_audio, int64_t n, int frame, float* d_out, void* stream) {
     MW_REQUIRE(d_audio && d_out && frame > 0 && n >= 0, "mw_frame_rms: bad argument");
     const int64_t n_frames = n / frame;

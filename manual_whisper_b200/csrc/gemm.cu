@@ -365,3 +365,33 @@ extern "C" mw_status mw_gemm_h16(const void* d_a, const void* d_w, const float* 
     a.batch = 1; a.M = M; a.N = N; a.K = K; a.gelu = gelu != 0; a.out_f32 = out_f32 != 0;
     return mw::gemm_launch(a, (cudaStream_t)stream);
 }
+
+extern "C" mw_status mw_gemm_general_h16(const void* d_a, int64_t a_row_stride, int64_t a_batch_stride, const void* d_w,
+                                          int64_t w_row_stride, const float* d_bias, const float* d_resid, int64_t res_batch_rows,
+                                          int64_t ld_res, void* d_out, int64_t out_batch_rows, int64_t out_row_off, int64_t ld_out,
+                                          int batch, int M, int N, int K, int gelu, int out_f32, void* stream) {
+    // shapes and strides first, then the pointers: a rejected call touches no memory
+    MW_REQUIRE(batch > 0 && M > 0 && N > 0 && K > 0 && N % 32 == 0 && K % 8 == 0,
+               "mw_gemm_general_h16: bad shape batch=%d M=%d N=%d K=%d (N %% 32 == 0, K %% 8 == 0)", batch, M, N, K);
+    MW_REQUIRE(a_row_stride > 0 && a_row_stride % 8 == 0 && a_batch_stride >= 0 && a_batch_stride % 8 == 0 &&
+               w_row_stride >= K && w_row_stride % 8 == 0,
+               "mw_gemm_general_h16: operand strides must be positive multiples of 8 (a_row_stride=%lld a_batch_stride=%lld "
+               "w_row_stride=%lld, K=%d)", (long long)a_row_stride, (long long)a_batch_stride, (long long)w_row_stride, K);
+    MW_REQUIRE(ld_out >= N && ld_out % 8 == 0 && out_row_off >= 0 && out_batch_rows >= 0 &&
+               (batch == 1 || out_batch_rows >= out_row_off + M),
+               "mw_gemm_general_h16: bad output geometry ld_out=%lld out_batch_rows=%lld out_row_off=%lld (N=%d M=%d)",
+               (long long)ld_out, (long long)out_batch_rows, (long long)out_row_off, N, M);
+    MW_REQUIRE(!d_resid || (ld_res >= N && ld_res % 4 == 0 && res_batch_rows >= 0),
+               "mw_gemm_general_h16: bad residual geometry ld_res=%lld res_batch_rows=%lld", (long long)ld_res,
+               (long long)res_batch_rows);
+    MW_REQUIRE(d_a && d_w && d_out, "mw_gemm_general_h16: null pointer");
+    MW_REQUIRE((uintptr_t)d_bias % 16 == 0 && (uintptr_t)d_resid % 16 == 0,
+               "mw_gemm_general_h16: bias and residual must be 16-byte aligned");
+    mw::GemmArgs a;
+    a.a = d_a; a.a_row_stride = a_row_stride; a.a_batch_stride = a_batch_stride;
+    a.w = d_w; a.w_row_stride = w_row_stride;
+    a.bias = d_bias; a.residual = d_resid; a.res_batch_rows = res_batch_rows; a.ld_res = ld_res;
+    a.out = d_out; a.out_batch_rows = out_batch_rows; a.out_row_off = out_row_off; a.ld_out = ld_out;
+    a.batch = batch; a.M = M; a.N = N; a.K = K; a.gelu = gelu != 0; a.out_f32 = out_f32 != 0;
+    return mw::gemm_launch(a, (cudaStream_t)stream);
+}

@@ -84,6 +84,46 @@ def test_step_entry_points_reject_bad_arguments_without_a_gpu(built_lib):
     assert cross(None, None, 2, 1, 1500, 6, 8, None, None) == 1 and b"null" in lib.mw_last_error()
 
 
+def test_building_block_entry_points_reject_bad_arguments_without_a_gpu(built_lib):
+    """mw_gemm_general_h16, mw_attention_general_h16 and mw_layernorm_mode check shapes, strides, column ranges and the mode
+    before any pointer: every call here has null pointers and is rejected up front."""
+    from manual_whisper_b200 import _lib
+    lib = _lib.load()
+
+    def gemm(ars=240, abs_=0, wrs=240, resid=None, rbr=0, ldr=0, obr=0, off=0, ldo=384, batch=1, M=3000, N=384, K=240):
+        return lib.mw_gemm_general_h16(None, ars, abs_, None, wrs, None, resid, rbr, ldr, None, obr, off, ldo, batch, M, N, K,
+                                       1, 0, None)
+
+    assert gemm() == 1 and b"null" in lib.mw_last_error()                           # a good conv1 geometry, null pointers
+    assert gemm(ars=80, abs_=3002 * 80, obr=3002, off=1, batch=3) == 1 and b"null" in lib.mw_last_error()
+    for bad in (dict(N=48), dict(K=236), dict(M=0), dict(batch=0), dict(ars=84), dict(ars=0), dict(abs_=-8), dict(wrs=232),
+                dict(ldo=376), dict(ldo=388), dict(off=-1), dict(batch=2, obr=3000, off=1), dict(resid=16, ldr=380),
+                dict(resid=16, ldr=386), dict(resid=16, ldr=384, rbr=-1)):
+        assert gemm(**bad) == 1, bad
+        assert b"null" not in lib.mw_last_error(), bad
+
+    def att(ldq=3 * 384, cq=0, ldkv=3 * 384, ck=384, cv=768, out_ld=384, B=2, Tq=1500, Tk=1500, H=6, lens=None):
+        return lib.mw_attention_general_h16(None, ldq, cq, None, ldkv, ck, cv, None, out_ld, B, Tq, Tk, H, lens, None)
+
+    assert att() == 1 and b"null" in lib.mw_last_error()
+    assert att(ldq=384, ldkv=768, ck=0, cv=384, Tq=223) == 1 and b"null" in lib.mw_last_error()
+    for bad in (dict(B=0), dict(Tq=0), dict(Tk=0), dict(H=0), dict(H=7), dict(cq=64 * 13), dict(cq=-64), dict(ck=-8),
+                dict(cv=768 + 64), dict(ldq=384 + 4), dict(cq=4), dict(out_ld=320), dict(out_ld=388),
+                dict(ldq=384, ldkv=768, ck=0, cv=384, Tq=223, lens=16)):
+        assert att(**bad) == 1, bad
+        assert b"null" not in lib.mw_last_error(), bad
+    assert att(H=7) == 1 and b"do not fit" in lib.mw_last_error()
+    assert att(Tq=223, lens=16) == 1 and b"Tq == Tk" in lib.mw_last_error()
+
+    ln = lib.mw_layernorm_mode
+    for mode, d in ((0, 2048), (1, 512), (2, 128), (3, 2048)):
+        assert ln(None, None, None, None, 7, d, mode, None) == 1 and b"null" in lib.mw_last_error()
+    for mode, d in ((1, 640), (2, 1024), (3, 2176), (0, 100), (3, 0), (4, 512), (-1, 512)):
+        assert ln(None, None, None, None, 7, d, mode, None) == 1, (mode, d)
+        assert b"null" not in lib.mw_last_error(), (mode, d)
+    assert ln(None, None, None, None, -1, 512, 3, None) == 1 and b"null" not in lib.mw_last_error()
+
+
 def test_sass_is_blackwell_native(built_lib):
     """tcgen05.mma -> UTCHMMA, tcgen05.ld -> LDTM, TMA -> UTMALDG must be present in the sm_100a SASS."""
     sass = subprocess.check_output(["cuobjdump", "-sass", str(built_lib)], text=True)

@@ -1,8 +1,12 @@
-"""Each tensor-core kernel pinned on its own against a plain PyTorch fp32 reference (through the C ABI)."""
+"""Each tensor-core kernel pinned on its own (through the C ABI).  The tcgen05 GEMM, the flash attention and LayerNorm are held
+to the per-element float64 bounds of tests/test_gpu_tensor_core_paths.py, whose checks these tests run at their shapes; the
+decode GEMM against a plain PyTorch fp32 reference."""
 import ctypes as C
 
 import pytest
 import torch
+
+from test_gpu_tensor_core_paths import MODES, check_gemm_contiguous, check_layernorm, check_self_attention
 
 pytestmark = pytest.mark.gpu
 
@@ -26,27 +30,8 @@ def _stream():
                                    (4096, 5120, 1280), (777, 256, 5120), (300, 64, 1024), (100, 32, 128)])
 @pytest.mark.parametrize("mode", ["plain", "bias_gelu", "bias_resid_f32"])
 def test_gemm(lib, M, N, K, mode):
-    from manual_whisper_b200 import _lib
-    dev = torch.device("cuda:0")
-    g = torch.Generator(device=dev).manual_seed(M * 7 + N)
-    a = (torch.randn(M, K, device=dev, generator=g) * 0.5).to(_h16())
-    w = (torch.randn(N, K, device=dev, generator=g) * 0.05).to(_h16())
-    bias = torch.randn(N, device=dev, generator=g) if mode != "plain" else None
-    res = torch.randn(M, N, device=dev, generator=g) if mode == "bias_resid_f32" else None
-    f32 = mode == "bias_resid_f32"
-    out = torch.empty(M, N, device=dev, dtype=torch.float32 if f32 else _h16())
-    _lib.check(lib.mw_gemm_h16(a.data_ptr(), w.data_ptr(), bias.data_ptr() if bias is not None else None,
-                                res.data_ptr() if res is not None else None, out.data_ptr(), M, N, K,
-                                int(mode == "bias_gelu"), int(f32), _stream()), "gemm")
-    ref = a.float() @ w.float().t()
-    if bias is not None:
-        ref = ref + bias
-    if mode == "bias_gelu":
-        ref = torch.nn.functional.gelu(ref)
-    if res is not None:
-        ref = ref + res
-    tol = 2e-4 * ref.abs().max().item() if f32 else 2 ** -8 * ref.abs().max().item() + 1e-3
-    assert (out.float() - ref).abs().max().item() <= tol
+    """The tcgen05 GEMM on contiguous operands against float64, element by element."""
+    check_gemm_contiguous(lib, M, N, K, mode)
 
 
 @pytest.mark.parametrize("R,N,K", [(32, 1280, 1280), (17, 384, 384), (64, 3840, 1280), (68, 1280, 5120), (128, 5120, 1280),
@@ -93,27 +78,14 @@ def test_gemm_rejects_bad_shapes(lib):
 
 @pytest.mark.parametrize("B,T,H", [(1, 128, 1), (1, 200, 2), (3, 1500, 6), (1, 1500, 20), (2, 77, 4)])
 def test_encoder_attention(lib, B, T, H):
-    from manual_whisper_b200 import _lib
-    dev = torch.device("cuda:0")
-    d = H * 64
-    g = torch.Generator(device=dev).manual_seed(T)
-    qkv = torch.randn(B * T, 3 * d, device=dev, generator=g).to(_h16())
-    out = torch.zeros(B * T, d, device=dev, dtype=_h16())
-    _lib.check(lib.mw_attention_h16(qkv.data_ptr(), out.data_ptr(), B, T, H, _stream()), "attention")
-    q, k, v = [t.float().view(B, T, H, 64).transpose(1, 2) for t in qkv.split(d, dim=1)]
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).transpose(1, 2).reshape(B * T, d)
-    assert (out.float() - ref).abs().max().item() < 2 ** -7 * ref.abs().max().item() + 2e-3
+    """The flash attention on packed qkv against float64 with random scores and with every score pattern of
+    tests/test_gpu_tensor_core_paths.py (lazy rescale at every key block, peaks at the first / last key, low, huge and
+    fp16-subnormal probabilities)."""
+    for mode in MODES:
+        check_self_attention(lib, B, T, H, mode)
 
 
 @pytest.mark.parametrize("rows,d", [(1, 128), (1000, 384), (37, 1280), (48000, 1280),
                                     (33, 512), (33, 640), (33, 1536), (33, 2048)])    # the MAXV boundaries of layernorm_launch
 def test_layernorm(lib, rows, d):
-    from manual_whisper_b200 import _lib
-    dev = torch.device("cuda:0")
-    g = torch.Generator(device=dev).manual_seed(d)
-    x = torch.randn(rows, d, device=dev, generator=g) * 3 + 1
-    gam, bet = torch.randn(d, device=dev, generator=g), torch.randn(d, device=dev, generator=g)
-    out = torch.empty(rows, d, device=dev, dtype=_h16())
-    _lib.check(lib.mw_layernorm(x.data_ptr(), gam.data_ptr(), bet.data_ptr(), out.data_ptr(), rows, d, _stream()), "ln")
-    ref = torch.nn.functional.layer_norm(x, (d,), gam, bet, 1e-5)
-    assert torch.equal(out, ref.to(_h16())) or (out.float() - ref).abs().max().item() <= 2 ** -8 * ref.abs().max().item()
+    check_layernorm(lib, rows, d)

@@ -221,7 +221,7 @@ mw_status mw_layernorm_mode(float* d_x, const float* d_gamma, const float* d_bet
                             void* stream);
 
 /* The decode step's own kernels (csrc/decoder.cu) on caller buffers, for tests/test_gpu_decode_step.py.  The launch path is
- * named by an argument; no A/B environment hook changes what these run.  They may allocate a few bytes and synchronise. */
+ * named by an argument.  They may allocate a few bytes and synchronise. */
 enum mw_step_path {
     MW_STEP_PATH_GREEDY = 0,        /* the step's routing in greedy search: tcgen05 decode GEMM from 96 rows, else mma.sync */
     MW_STEP_PATH_BEAM = 1,          /* the step's routing of the layer projections in beam search: mma.sync kernels only */

@@ -331,14 +331,11 @@ bool decode_gemm_supported(int ldx, int ldw, int R, int N, int K) {
 }
 
 // split-K factor: enough CTAs to spread a small weight matrix over the machine, at least two 64-wide k-blocks per CTA
-static int dg_pick_ks(int tiles_m, int nkb, int R, bool hooks) {
-    static const int forced_env = [] { const char* e = getenv("MW_DG_KS"); return e ? atoi(e) : 0; }();
-    const int forced = hooks ? forced_env : 0;
+static int dg_pick_ks(int tiles_m, int nkb) {
     int ks = 1;
     for (int c : {2, 4, 8}) {
-        if (forced ? c <= forced : (tiles_m * c <= 160 && nkb / c >= 2)) ks = c;
+        if (tiles_m * c <= 160 && nkb / c >= 2) ks = c;
     }
-    while (ks > 1 && (nkb < ks || ((R + ks - 1) / ks) < 1)) ks >>= 1;
     return ks;
 }
 
@@ -346,7 +343,7 @@ static unsigned long long* g_dg_dbg = nullptr;
 void decode_gemm_set_debug(unsigned long long* d_stamps) { g_dg_dbg = d_stamps; }
 
 mw_status decode_gemm_launch(const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
-                             int ldo, int R, int N, int K, int flags, cudaStream_t st, bool hooks) {
+                             int ldo, int R, int N, int K, int flags, cudaStream_t st) {
     MW_REQUIRE(decode_gemm_supported(ldx, ldw, R, N, K), "decode gemm: unsupported shape R=%d N=%d K=%d", R, N, K);
     MW_REQUIRE(((uintptr_t)X % 16 == 0) && ((uintptr_t)W % 16 == 0), "decode gemm: operands must be 16-byte aligned");
     const DgLayout L = dg_layout(R);
@@ -368,7 +365,7 @@ mw_status decode_gemm_launch(const void* X, int ldx, const void* W, int ldw, con
         if (s != MW_OK) return s;
     }
     DgParams p;
-    p.R = R; p.N = N; p.nkb = nkb; p.ks = dg_pick_ks(tiles_m, nkb, R, hooks);
+    p.R = R; p.N = N; p.nkb = nkb; p.ks = dg_pick_ks(tiles_m, nkb);
     p.bias = bias; p.resid = resid; p.out = out; p.ldo = ldo; p.flags = flags; p.dbg = g_dg_dbg;
     switch (p.ks) {
         case 1: return dg_launch<1>(tw, tx, p, tiles_m, st);

@@ -78,9 +78,7 @@ struct DecoderState {
     // host side
     mw::DecCtl* h_ctl = nullptr;         // pinned [2]
     cudaStream_t cap_stream = nullptr;
-    bool use_prio = false;
     int parts_epoch = 0;
-    int prio_low = 0;
     cudaEvent_t ev[2] = {nullptr, nullptr};
     // step graphs are specific to (rows, beam): a small cache keeps the last few shapes (full batches and the short
     // last batch of a recording alternate) so they are not re-captured on every call
@@ -133,8 +131,6 @@ skinny_gemm_kernel(const mw_h* __restrict__ X, int ldx, const mw_h* __restrict__
                    const float* __restrict__ bias, const float* resid, void* out, int ldo, int R, int N, int K,
                    int flags) {
     __shared__ float red[8][32][17];
-    pdl_trigger();
-    pdl_wait();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int g = lane >> 2, q = lane & 3;
     const int n0 = blockIdx.x * 16, r0 = blockIdx.y * 32;
@@ -200,7 +196,6 @@ skinny_gemm_rows16_kernel(const mw_h* __restrict__ X, int ldx, const mw_h* __res
     // WT = 16-row weight tiles per CTA.  Every CTA re-reads the whole X block [32, K] from L2, so with one tile the L2->SM
     // traffic is 3x the HBM traffic and caps several batches in flight at ~3.3 TB/s of weights; two tiles halve the X share.
     __shared__ float red[NW][32][WT * 16 + 1];
-    pdl_trigger();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int g = lane >> 2, q = lane & 3;
     const int n0 = blockIdx.x * (16 * WT), r0 = blockIdx.y * 32;
@@ -216,7 +211,7 @@ skinny_gemm_rows16_kernel(const mw_h* __restrict__ X, int ldx, const mw_h* __res
             ahi[wt][i] = ldg_stream(wb + i * 32);
         }
     }
-    pdl_wait();        // the weights above are in flight; X (and resid, out) belong to the chain
+    // the whole weight slice is in flight before the first X load is issued
     const mw_h* xr[4];
 #pragma unroll
     for (int t = 0; t < 4; ++t) xr[t] = X + (int64_t)min(r0 + t * 8 + g, R - 1) * ldx + k_start;
@@ -418,7 +413,6 @@ skinny_gemm_rows32_khalf_kernel(const mw_h* __restrict__ X, int ldx, const mw_h*
     // WT = 2 weight tiles per CTA; WT = 1 (a lone batch, mw_set_solo) doubles the CTAs and halves the bytes each waits for -
     // per output element the K order and the reduction are the same, so both give the same bits
     __shared__ float red[NW / 2][32][WT * 16 + 1];
-    pdl_trigger();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int g = lane >> 2, q = lane & 3;
     const int n0 = blockIdx.x * (16 * WT), r0 = blockIdx.y * 32;
@@ -443,7 +437,7 @@ skinny_gemm_rows32_khalf_kernel(const mw_h* __restrict__ X, int ldx, const mw_h*
                 ahi[wt][i] = ldg_stream(wb + i * 32);
             }
         }
-        if (h == 0) pdl_wait();        // first half of the weights in flight; X belongs to the chain
+        // this half's weights are in flight before its X loads are issued
 #pragma unroll
         for (int i = 0; i < KB; ++i) {
             uint4 b[4];
@@ -494,34 +488,12 @@ skinny_gemm_rows32_khalf_kernel(const mw_h* __restrict__ X, int ldx, const mw_h*
     }
 }
 
-// Which kernel a decode-step projection runs.  SK_STEP is the step's own routing, A/B hooks included (read once per process);
-// SK_ROUTE is the same routing with every hook at its default; the others force one kernel (mw_step_projection_h16).
-enum SkPath { SK_STEP, SK_ROUTE, SK_ROWS16_WT1, SK_ROWS16_WT2, SK_KHALF_WT1, SK_KHALF_WT2, SK_GENERIC, SK_LN_FUSED, SK_LN_SEPARATE };
+// Which kernel a decode-step projection runs.  SK_ROUTE is the step's own routing; the others force one kernel
+// (mw_step_projection_h16).
+enum SkPath { SK_ROUTE, SK_ROWS16_WT1, SK_ROWS16_WT2, SK_KHALF_WT1, SK_KHALF_WT2, SK_GENERIC, SK_LN_FUSED, SK_LN_SEPARATE };
 
-struct SkHooks {
-    bool one_tile;      // MW_SKINNY_WT=1: one weight tile per CTA in the mma.sync projections
-    bool no_khalf;      // MW_SKINNY_KHALF=0: no K-halved kernel
-    int khalf_wt;       // MW_KHALF_WT: 0 = by mw_set_solo, 1 / 2 = forced
-    int dg_min_rows;    // MW_DG_MIN_ROWS: rows from which the tcgen05 decode GEMM takes over
-    int ln_fuse;        // MW_LN_FUSE: -1 = by mw_set_solo, 0 never, 1 always
-    bool prefetch;      // MW_PREFETCH=0 switches the L2 prefetch of the next projection's weights off
-};
-constexpr SkHooks SK_DEFAULT_HOOKS = {false, false, 0, 96, -1, true};
-const SkHooks& sk_env_hooks() {
-    static const SkHooks h = [] {
-        SkHooks v = SK_DEFAULT_HOOKS;
-        const char* e;
-        if ((e = getenv("MW_SKINNY_WT"))) v.one_tile = e[0] == '1';
-        if ((e = getenv("MW_SKINNY_KHALF"))) v.no_khalf = e[0] == '0';
-        if ((e = getenv("MW_KHALF_WT"))) v.khalf_wt = atoi(e);
-        if ((e = getenv("MW_DG_MIN_ROWS"))) v.dg_min_rows = atoi(e);
-        if ((e = getenv("MW_LN_FUSE"))) v.ln_fuse = atoi(e);
-        if ((e = getenv("MW_PREFETCH"))) v.prefetch = e[0] != '0';
-        return v;
-    }();
-    return h;
-}
-const SkHooks& sk_hooks(SkPath path) { return path == SK_STEP ? sk_env_hooks() : SK_DEFAULT_HOOKS; }
+// rows from which the tcgen05 decode GEMM takes over the projections the step routes to it (see skinny_gemm)
+constexpr int DG_MIN_ROWS = 96;
 
 // The tuned projections of skinny_gemm (its MW_SK table): warps per CTA for K = KB * NW * 32, 0 when K has no entry.
 // The K-halved kernel serves the 16-warp entries; two weight tiles fit the registers for KB <= 5 with at most 8 warps.
@@ -542,8 +514,7 @@ mw_status launch_rows16(const void* X, int ldx, const void* W, int ldw, const fl
                         int ldo, int R, int N, int K, int flags, cudaStream_t st, const char* pf, int pf_lines, bool solo,
                         SkPath path) {
     constexpr int WT = (NW <= 8 && KB <= 5) ? 2 : 1;          // two weight tiles where the registers allow it
-    const SkHooks& hk = sk_hooks(path);
-    const bool routed = path == SK_STEP || path == SK_ROUTE;
+    const bool routed = path == SK_ROUTE;
     if ((path == SK_KHALF_WT1 || path == SK_KHALF_WT2) && !(NW == 16 && KB % 2 == 0 && KB / 2 <= 5)) {
         set_error("skinny gemm: no K-halved kernel for K=%d", K);
         return MW_ERR_UNSUPPORTED;
@@ -553,29 +524,29 @@ mw_status launch_rows16(const void* X, int ldx, const void* W, int ldw, const fl
         return MW_ERR_UNSUPPORTED;
     }
     if constexpr (NW == 16 && KB % 2 == 0 && KB / 2 <= 5) {
-        if ((routed && !hk.one_tile && !hk.no_khalf) || path == SK_KHALF_WT1 || path == SK_KHALF_WT2) {
-            const bool one = routed ? (hk.khalf_wt == 1 || (hk.khalf_wt == 0 && solo)) : path == SK_KHALF_WT1;
+        if (routed || path == SK_KHALF_WT1 || path == SK_KHALF_WT2) {
+            const bool one = routed ? solo : path == SK_KHALF_WT1;
             if (one) {       // a lone batch: 3.87 -> 3.76 ms per single-stream step
                 dim3 grid(ceil_div(N, 16), ceil_div(R, 32));
-                launch_chained(skinny_gemm_rows32_khalf_kernel<KB / 2, NW, 1>, grid, dim3(NW * 32), 0, st, (const mw_h*)X, ldx,
-                               (const mw_h*)W, ldw, bias, resid, out, ldo, R, N, K, flags, pf, pf_lines);
+                skinny_gemm_rows32_khalf_kernel<KB / 2, NW, 1><<<grid, NW * 32, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias,
+                                                                                        resid, out, ldo, R, N, K, flags, pf, pf_lines);
             } else {
                 dim3 grid(ceil_div(N, 32), ceil_div(R, 32));
-                launch_chained(skinny_gemm_rows32_khalf_kernel<KB / 2, NW, 2>, grid, dim3(NW * 32), 0, st, (const mw_h*)X, ldx,
-                               (const mw_h*)W, ldw, bias, resid, out, ldo, R, N, K, flags, pf, pf_lines);
+                skinny_gemm_rows32_khalf_kernel<KB / 2, NW, 2><<<grid, NW * 32, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias,
+                                                                                        resid, out, ldo, R, N, K, flags, pf, pf_lines);
             }
             MW_LAUNCH_CHECK();
             return MW_OK;
         }
     }
-    if (WT == 2 && ((routed && !hk.one_tile) || path == SK_ROWS16_WT2)) {
+    if (WT == 2 && (routed || path == SK_ROWS16_WT2)) {
         dim3 grid(ceil_div(N, 32), ceil_div(R, 32));
-        launch_chained(skinny_gemm_rows16_kernel<KB, NW, WT>, grid, dim3(NW * 32), 0, st, (const mw_h*)X, ldx, (const mw_h*)W, ldw,
-                       bias, resid, out, ldo, R, N, K, flags, pf, pf_lines);
+        skinny_gemm_rows16_kernel<KB, NW, WT><<<grid, NW * 32, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias, resid, out, ldo,
+                                                                       R, N, K, flags, pf, pf_lines);
     } else {
         dim3 grid(ceil_div(N, 16), ceil_div(R, 32));
-        launch_chained(skinny_gemm_rows16_kernel<KB, NW, 1>, grid, dim3(NW * 32), 0, st, (const mw_h*)X, ldx, (const mw_h*)W, ldw,
-                       bias, resid, out, ldo, R, N, K, flags, pf, pf_lines);
+        skinny_gemm_rows16_kernel<KB, NW, 1><<<grid, NW * 32, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias, resid, out, ldo,
+                                                                      R, N, K, flags, pf, pf_lines);
     }
     MW_LAUNCH_CHECK();
     return MW_OK;
@@ -584,19 +555,18 @@ mw_status launch_rows16(const void* X, int ldx, const void* W, int ldw, const fl
 // `next_w` / `next_bytes`: the weight matrix of the projection that follows this one in the step (prefetched into L2)
 mw_status skinny_gemm(const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
                       int ldo, int R, int N, int K, int flags, cudaStream_t st, bool allow_dg = true,
-                      const void* next_w = nullptr, int64_t next_bytes = 0, bool solo = false, SkPath path = SK_STEP) {
-    const SkHooks& hk = sk_hooks(path);
-    const bool routed = path == SK_STEP || path == SK_ROUTE;
-    const char* pf = hk.prefetch ? (const char*)next_w : nullptr;
+                      const void* next_w = nullptr, int64_t next_bytes = 0, bool solo = false, SkPath path = SK_ROUTE) {
+    const bool routed = path == SK_ROUTE;
+    const char* pf = (const char*)next_w;
     const int pf_lines = pf ? (int)(next_bytes / 128) : 0;
-    // R >= MW_DG_MIN_ROWS rows (merged greedy batches): the weight-stationary tcgen05 kernel (decode_gemm.cu) streams W once
+    // R >= DG_MIN_ROWS rows (merged greedy batches): the weight-stationary tcgen05 kernel (decode_gemm.cu) streams W once
     // for all rows; the mma.sync kernels below re-read it per 32-row block (from L2 after the first block) and stay in charge
     // of the 32-row batches they were tuned on and of beam search, where they measured faster (DESIGN.md section 4: a decode
     // step is a chain of ~360 latency-bound launches, so bytes saved do not buy time unless the launch is also shorter).
     // The step passes allow_dg = (beam <= 1) for the layer projections; the vocabulary projection (enqueue_logits) keeps the
     // default, so at R >= 96 rows it runs on the decode GEMM in beam search as well.
-    if (routed && allow_dg && R >= hk.dg_min_rows && decode_gemm_supported(ldx, ldw, R, N, K))
-        return decode_gemm_launch(X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st, path == SK_STEP);
+    if (routed && allow_dg && R >= DG_MIN_ROWS && decode_gemm_supported(ldx, ldw, R, N, K))
+        return decode_gemm_launch(X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st);
     if (!routed && path != SK_GENERIC && !sk_table_warps(K)) {
         set_error("skinny gemm: no tuned kernel for K=%d (the generic kernel serves it)", K);
         return MW_ERR_UNSUPPORTED;
@@ -616,8 +586,7 @@ mw_status skinny_gemm(const void* X, int ldx, const void* W, int ldw, const floa
     MW_SK(1, 8);    // 256
 #undef MW_SK
     dim3 grid(ceil_div(N, 16), ceil_div(R, 32));
-    launch_chained(skinny_gemm_kernel, grid, dim3(256), 0, st, (const mw_h*)X, ldx, (const mw_h*)W, ldw, bias, resid, out, ldo, R, N, K,
-                   flags);
+    skinny_gemm_kernel<<<grid, 256, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias, resid, out, ldo, R, N, K, flags);
     MW_LAUNCH_CHECK();
     return MW_OK;
 }
@@ -625,8 +594,6 @@ mw_status skinny_gemm(const void* X, int ldx, const void* W, int ldw, const floa
 // ------------------------------------------------------------------------------------------------
 __global__ void embed_kernel(const int* __restrict__ cur_tok, const mw_h* __restrict__ emb,
                              const float* __restrict__ pos_emb, const DecCtl* __restrict__ ctl, float* __restrict__ x, int d) {
-    pdl_trigger();
-    pdl_wait();
     const int r = blockIdx.x;
     const int tok = cur_tok[r];
     const int pos = ctl->pos;
@@ -644,16 +611,15 @@ __global__ void embed_kernel(const int* __restrict__ cur_tok, const mw_h* __rest
 // 16-bit operand twice in the plain kernels costs nothing at eight streams.)
 mw_status skinny_gemm_ln(const float* x, const float* gamma, const float* beta, void* ln_buf, const void* W, const float* bias,
                          void* out, int ldo, int R, int N, int K, int flags, cudaStream_t st, bool allow_dg, const void* next_w,
-                         int64_t next_bytes, bool solo, SkPath path = SK_STEP) {
-    const SkHooks& hk = sk_hooks(path);
-    const bool fuse = path == SK_LN_FUSED || ((path == SK_STEP || path == SK_ROUTE) && (hk.ln_fuse < 0 ? solo : hk.ln_fuse != 0));
-    const bool to_dg = path != SK_LN_FUSED && allow_dg && R >= hk.dg_min_rows && decode_gemm_supported(K, K, R, N, K);
+                         int64_t next_bytes, bool solo, SkPath path = SK_ROUTE) {
+    const bool fuse = path == SK_LN_FUSED || (path == SK_ROUTE && solo);
+    const bool to_dg = path != SK_LN_FUSED && allow_dg && R >= DG_MIN_ROWS && decode_gemm_supported(K, K, R, N, K);
     if (path == SK_LN_FUSED && (!sk_has_ln_fused(K) || (flags & SK_FLAG_F32))) {
         set_error("skinny gemm: no fused LayerNorm projection for K=%d%s", K, (flags & SK_FLAG_F32) ? " with fp32 output" : "");
         return MW_ERR_UNSUPPORTED;
     }
     if (fuse && !to_dg && !(flags & SK_FLAG_F32)) {
-        const char* pf = hk.prefetch ? (const char*)next_w : nullptr;
+        const char* pf = (const char*)next_w;
         const int pf_lines = pf ? (int)(next_bytes / 128) : 0;
 #define MW_SKLN(kb, nw) if (K == kb * nw * 32) return launch_ln_rows16<kb, nw>(x, gamma, beta, W, K, bias, out, ldo, R, N, flags, st, pf, pf_lines)
         MW_SKLN(5, 8);    // 1280  (large)
@@ -667,8 +633,7 @@ mw_status skinny_gemm_ln(const float* x, const float* gamma, const float* beta, 
     }
     mw_status r = layernorm_launch(x, gamma, beta, ln_buf, R, K, st);
     if (r != MW_OK) return r;
-    return skinny_gemm(ln_buf, K, W, K, bias, nullptr, out, ldo, R, N, K, flags, st, allow_dg, next_w, next_bytes, false,
-                       path == SK_STEP ? SK_STEP : SK_ROUTE);
+    return skinny_gemm(ln_buf, K, W, K, bias, nullptr, out, ldo, R, N, K, flags, st, allow_dg, next_w, next_bytes, false, SK_ROUTE);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -695,8 +660,6 @@ decode_attn_kernel(const mw_h* __restrict__ q, int ldq,
     extern __shared__ float sc[];          // scores [n_keys] + reduction scratch
     __shared__ float red[4][64];
     __shared__ float red_s[8];
-    pdl_trigger();
-    pdl_wait();
     const int h = blockIdx.x, r = blockIdx.y;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     constexpr int UNR = SELF ? 4 : 8;             // independent 16-byte loads in flight per thread
@@ -833,8 +796,6 @@ cross_attn_stream_kernel(const mw_h* __restrict__ q, int ldq, const mw_h* __rest
                          mw_h* __restrict__ out, int ldo, const char* pf, int pf_lines) {
     __shared__ float part_acc[16][64];
     __shared__ float part_m[16], part_l[16];
-    pdl_trigger();
-    pdl_wait();
     const int h = blockIdx.x, r = blockIdx.y;
     const int key_lo = 0, key_hi = n_keys;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -934,8 +895,6 @@ cross_attn_grouped_kernel(const mw_h* __restrict__ q, int ldq, const mw_h* __res
     __shared__ float red[4][G][64];
     __shared__ float red_s[G][8];
     constexpr int UNR = 4;
-    pdl_trigger();
-    pdl_wait();
     const int h = blockIdx.x, b = blockIdx.y;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int lg = lane & 7, kq = lane >> 3;
@@ -1071,7 +1030,7 @@ mw_status launch_cross_grouped(const mw_h* q, int ldq, const mw_h* k, const mw_h
     MW_REQUIRE(smem <= 96 * 1024, "cross attention: %zu bytes of scores exceed shared memory", smem);
     static PerDeviceOnce attr_once;
     MW_CUDA_CHECK(attr_once.run([&] { return cudaFuncSetAttribute(cross_attn_grouped_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); }));
-    launch_chained(cross_attn_grouped_kernel<G>, dim3(n_heads, B), dim3(128), smem, st, q, ldq, k, v, key_stride, n_keys, out, ldo);
+    cross_attn_grouped_kernel<G><<<dim3(n_heads, B), 128, smem, st>>>(q, ldq, k, v, key_stride, n_keys, out, ldo);
     MW_LAUNCH_CHECK();
     return MW_OK;
 }
@@ -1226,8 +1185,6 @@ __global__ void __launch_bounds__(SEL_THREADS)
 select_greedy_kernel(float* logits, int V, const GenOptsDev* __restrict__ opts, const uint8_t* __restrict__ sup,
                      const uint8_t* __restrict__ beg, int* tokens, int* gen_len, int* done, float* cum, int* last_ts,
                      int* cur_tok, DecCtl* ctl, int max_new) {
-    pdl_trigger();
-    pdl_wait();
     const int r = blockIdx.x;
     const GenOptsDev o = *opts;
     float* lg = logits + (int64_t)r * V;
@@ -1263,8 +1220,6 @@ select_greedy_kernel(float* logits, int V, const GenOptsDev* __restrict__ opts, 
 __global__ void advance_forced_kernel(const int* __restrict__ forced, int per_row_stride, int n_forced, int* cur_tok,
                                       DecCtl* ctl, int R) {
     // single CTA: every thread reads ctl->step before thread 0 advances it
-    pdl_trigger();
-    pdl_wait();
     const int next = ctl->step + 1;
     if (next < n_forced)
         for (int r = threadIdx.x; r < R; r += blockDim.x) cur_tok[r] = forced[(int64_t)r * per_row_stride + next];
@@ -1283,8 +1238,6 @@ beam_candidates_kernel(float* logits, int V, const GenOptsDev* __restrict__ opts
                        DecCtl* ctl) {
     __shared__ ValIdx s_c[SEL_THREADS / 32];
     __shared__ ValIdx s_pick;
-    pdl_trigger();
-    pdl_wait();
     const int r = blockIdx.x;
     const GenOptsDev o = *opts;
     float* lg = logits + (int64_t)r * V;
@@ -1354,8 +1307,6 @@ __global__ void beam_update_kernel(const GenOptsDev* __restrict__ opts, const fl
                                    const int* __restrict__ idx_in, int* idx_out, int ctx,
                                    int* fin_count, float* fin_score, int* fin_len, int* fin_tok, int* active,
                                    int* cur_tok, DecCtl* ctl, int B, int max_new) {
-    pdl_trigger();
-    pdl_wait();
     const GenOptsDev o = *opts;
     const int k = o.beam, nc = 2 * k;
     const int b = blockIdx.x;
@@ -1551,19 +1502,7 @@ mw_status decoder_state_create(mw_model* m) {
     A((void**)&s->active, B * 4, true);
     if (st != MW_OK) return st;
     MW_CUDA_CHECK(cudaMallocHost((void**)&s->h_ctl, 2 * sizeof(DecCtl)));
-    // Experiment hook, OFF unless MW_PRIO=1: capture the step graphs on a HIGH-priority stream and launch the one
-    // bandwidth-hungry kernel of the step (cross-attention) at the LOWEST priority, so that with several batches in flight the
-    // short latency-bound kernels of one batch get SM slots ahead of another batch's queued cross-attention CTAs.  Measured
-    // on the real generate loop (scripts/gpu_generate_concurrent.py): no change (451.2 vs 451.4 ms per batch) - the kernel
-    // classes of concurrent batches already time-slice additively, DESIGN.md section 4.
-    {
-        int least = 0, greatest = 0;
-        MW_CUDA_CHECK(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-        const char* e = getenv("MW_PRIO");
-        s->use_prio = (e && e[0] == '1') && greatest < least;
-        s->prio_low = least;
-        MW_CUDA_CHECK(cudaStreamCreateWithPriority(&s->cap_stream, cudaStreamNonBlocking, s->use_prio ? greatest : least));
-    }
+    MW_CUDA_CHECK(cudaStreamCreateWithFlags(&s->cap_stream, cudaStreamNonBlocking));
     for (int i = 0; i < 2; ++i) MW_CUDA_CHECK(cudaEventCreateWithFlags(&s->ev[i], cudaEventDisableTiming));
     MW_CUDA_CHECK(cudaFuncSetAttribute(decode_attn_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
     return MW_OK;
@@ -1617,8 +1556,7 @@ mw_status enqueue_layers(mw_model* m, int R, int beam, int idx_phase, cudaStream
     const int d = c.d_model, ctx = c.n_text_ctx, T = c.n_audio_ctx;
     mw_status r;
     if (parts & PART_EMBED) {
-        launch_chained(embed_kernel, dim3(R), dim3(128), 0, st, s->cur_tok, (const mw_h*)m->gw(MW_DEC_EMB), (const float*)m->gw(MW_DEC_POS),
-                       s->ctl, s->x, d);
+        embed_kernel<<<R, 128, 0, st>>>(s->cur_tok, (const mw_h*)m->gw(MW_DEC_EMB), (const float*)m->gw(MW_DEC_POS), s->ctl, s->x, d);
         MW_LAUNCH_CHECK();
     }
     const int* idx = beam > 1 ? s->self_idx[idx_phase] : nullptr;
@@ -1629,8 +1567,7 @@ mw_status enqueue_layers(mw_model* m, int R, int beam, int idx_phase, cudaStream
         const bool dg = beam <= 1;
         const int64_t dd = (int64_t)d * d * 2, df = (int64_t)d * c.ffn * 2;          // bytes of a d x d / d x ffn weight matrix
         const void* next_qkv = l + 1 < c.dec_layers ? m->dlw(l + 1, MW_DL_WQKV) : nullptr;
-        static const bool pf_on = [] { const char* e = getenv("MW_PREFETCH"); return !(e && e[0] == '0'); }();
-        const char* pf_xo = (pf_on && GM) ? (const char*)W(MW_DL_WXO) : nullptr;
+        const char* pf_xo = GM ? (const char*)W(MW_DL_WXO) : nullptr;
         if (LN && GM) {
             if ((r = skinny_gemm_ln(s->x, F(MW_DL_LN1_G), F(MW_DL_LN1_B), s->ln, W(MW_DL_WQKV), F(MW_DL_BQKV), s->qkv, 3 * d, R, 3 * d, d, 0,
                                     st, dg, W(MW_DL_WO), dd, s->solo)) != MW_OK) return r;
@@ -1642,8 +1579,8 @@ mw_status enqueue_layers(mw_model* m, int R, int beam, int idx_phase, cudaStream
             mw_h* kc = s->k_self + (int64_t)l * s->R_max * ctx * d;
             mw_h* vc = s->v_self + (int64_t)l * s->R_max * ctx * d;
             dim3 grid(c.n_heads, R);
-            launch_chained(decode_attn_kernel<true>, grid, dim3(128), ctx * sizeof(float), st, s->qkv, 3 * d, kc, vc, d, ctx, idx, ctx,
-                           s->ctl, 0, 1, s->qkv + d, s->qkv + 2 * d, 3 * d, s->att, d, 0);
+            decode_attn_kernel<true><<<grid, 128, ctx * sizeof(float), st>>>(s->qkv, 3 * d, kc, vc, d, ctx, idx, ctx, s->ctl, 0, 1, s->qkv + d,
+                                                                            s->qkv + 2 * d, 3 * d, s->att, d, 0);
             MW_LAUNCH_CHECK();
         }
         if (GM && (r = skinny_gemm(s->att, d, W(MW_DL_WO), d, F(MW_DL_BO), s->x, s->x, d, R, d, d, SK_FLAG_F32, st, dg, W(MW_DL_WXQ), dd)) != MW_OK) return r;
@@ -1667,28 +1604,12 @@ mw_status enqueue_layers(mw_model* m, int R, int beam, int idx_phase, cudaStream
                 if (r != MW_OK) return r;
             } else {
                 dim3 grid(c.n_heads, R);
-                if (s->use_prio) {
-                    cudaLaunchConfig_t cfg = {};
-                    cfg.gridDim = grid; cfg.blockDim = dim3(128, 1, 1); cfg.dynamicSmemBytes = 0; cfg.stream = st;
-                    cudaLaunchAttribute attr[1];
-                    attr[0].id = cudaLaunchAttributePriority;
-                    attr[0].val.priority = s->prio_low;
-                    cfg.attrs = attr; cfg.numAttrs = 1;
-                    MW_CUDA_CHECK(cudaLaunchKernelEx(&cfg, cross_attn_stream_kernel<4>, (const mw_h*)s->qx, d, (const mw_h*)kv,
-                                                     (const mw_h*)(kv + d), (int64_t)(2 * d), T, s->att, d, pf_xo, (int)(dd / 128)));
-                    count_launch();
-                } else {
-                    // under-filled grid (fewer CTAs than 3 per SM): more loads in flight per CTA, same arithmetic
-                    static const int unr_env = [] { const char* e = getenv("MW_XATTN_UNR"); return e ? atoi(e) : 0; }();   // A/B hook
-                    const bool deep = unr_env ? unr_env == 8 : (int)(grid.x * grid.y) <= 3 * device_sm_count();
-                    if (deep)
-                        launch_chained(cross_attn_stream_kernel<8>, grid, dim3(128), 0, st, s->qx, d, kv, kv + d, 2 * d, T, s->att, d, pf_xo,
-                                       (int)(dd / 128));
-                    else
-                        launch_chained(cross_attn_stream_kernel<4>, grid, dim3(128), 0, st, s->qx, d, kv, kv + d, 2 * d, T, s->att, d, pf_xo,
-                                       (int)(dd / 128));
-                    MW_LAUNCH_CHECK();
-                }
+                // under-filled grid (fewer CTAs than 3 per SM): more loads in flight per CTA, same arithmetic
+                if ((int)(grid.x * grid.y) <= 3 * device_sm_count())
+                    cross_attn_stream_kernel<8><<<grid, 128, 0, st>>>(s->qx, d, kv, kv + d, 2 * d, T, s->att, d, pf_xo, (int)(dd / 128));
+                else
+                    cross_attn_stream_kernel<4><<<grid, 128, 0, st>>>(s->qx, d, kv, kv + d, 2 * d, T, s->att, d, pf_xo, (int)(dd / 128));
+                MW_LAUNCH_CHECK();
             }
         }
         if (GM && (r = skinny_gemm(s->att, d, W(MW_DL_WXO), d, F(MW_DL_BXO), s->x, s->x, d, R, d, d, SK_FLAG_F32, st, dg, W(MW_DL_W1), df)) != MW_OK) return r;
@@ -1718,18 +1639,19 @@ mw_status enqueue_select(mw_model* m, int B, int beam, int phase, cudaStream_t s
     DecoderState* s = m->dec;
     const int R = B * beam;
     if (beam <= 1) {
-        launch_chained(select_greedy_kernel, dim3(R), dim3(SEL_THREADS), 0, st, s->logits, c.vocab, s->opts, s->sup_mask, s->begin_mask,
-                       s->tokens[0], s->gen_len, s->done, s->cum, s->last_ts[0], s->cur_tok, s->ctl, s->max_new);
+        select_greedy_kernel<<<R, SEL_THREADS, 0, st>>>(s->logits, c.vocab, s->opts, s->sup_mask, s->begin_mask, s->tokens[0], s->gen_len,
+                                                       s->done, s->cum, s->last_ts[0], s->cur_tok, s->ctl, s->max_new);
         MW_LAUNCH_CHECK();
         return MW_OK;
     }
-    launch_chained(beam_candidates_kernel, dim3(R), dim3(SEL_THREADS), 0, st, s->logits, c.vocab, s->opts, s->sup_mask, s->begin_mask,
-                   s->tokens[phase], s->gen_len, s->last_ts[phase], s->cand_val, s->cand_idx, s->row_lse, s->max_new, s->ctl);
+    beam_candidates_kernel<<<R, SEL_THREADS, 0, st>>>(s->logits, c.vocab, s->opts, s->sup_mask, s->begin_mask, s->tokens[phase],
+                                                      s->gen_len, s->last_ts[phase], s->cand_val, s->cand_idx, s->row_lse, s->max_new,
+                                                      s->ctl);
     MW_LAUNCH_CHECK();
-    launch_chained(beam_update_kernel, dim3(B), dim3(128), 0, st, s->opts, s->cand_val, s->cand_idx, s->row_lse, s->tokens[phase],
-                   s->tokens[phase ^ 1], s->gen_len, s->cum, s->last_ts[phase], s->last_ts[phase ^ 1], s->self_idx[phase],
-                   s->self_idx[phase ^ 1], c.n_text_ctx, s->fin_count, s->fin_score, s->fin_len, s->fin_tok, s->active, s->cur_tok,
-                   s->ctl, B, s->max_new);
+    beam_update_kernel<<<B, 128, 0, st>>>(s->opts, s->cand_val, s->cand_idx, s->row_lse, s->tokens[phase], s->tokens[phase ^ 1],
+                                          s->gen_len, s->cum, s->last_ts[phase], s->last_ts[phase ^ 1], s->self_idx[phase],
+                                          s->self_idx[phase ^ 1], c.n_text_ctx, s->fin_count, s->fin_score, s->fin_len, s->fin_tok,
+                                          s->active, s->cur_tok, s->ctl, B, s->max_new);
     MW_LAUNCH_CHECK();
     return MW_OK;
 }
@@ -1835,7 +1757,7 @@ mw_status batched_prefill(mw_model* m, int B, int beam, int Pm, cudaStream_t st)
     return MW_OK;
 }
 
-std::atomic<int> g_step_parts{[] { const char* e = getenv("MW_STEP_PARTS"); return e ? atoi(e) : (int)PART_ALL; }()};
+std::atomic<int> g_step_parts{PART_ALL};
 std::atomic<int> g_step_parts_epoch{0};
 
 mw_status ensure_graphs(mw_model* m, int B, int beam) {
@@ -1861,13 +1783,13 @@ mw_status ensure_graphs(mw_model* m, int B, int beam) {
     r = capture_graph(s, &s->graphs.prefill, &s->graphs.n_prefill, [&](cudaStream_t st) -> mw_status {
         mw_status q = enqueue_layers(m, R, beam, 0, st);
         if (q != MW_OK) return q;
-        launch_chained(advance_forced_kernel, dim3(1), dim3(256), 0, st, s->prompt, 0, 1 << 30, s->cur_tok, s->ctl, R);
+        advance_forced_kernel<<<1, 256, 0, st>>>(s->prompt, 0, 1 << 30, s->cur_tok, s->ctl, R);
         MW_LAUNCH_CHECK();
         return MW_OK;
     });
     if (r != MW_OK) { destroy_graph_entry(s->graphs); return r; }
     for (int phase = 0; phase < (beam > 1 ? 2 : 1); ++phase) {
-        // measurement only (mw_debug_step_parts / MW_STEP_PARTS; ids are then meaningless): kernel classes kept in the step graph
+        // measurement only (mw_debug_step_parts; ids are then meaningless): kernel classes kept in the step graph
         const int step_parts = g_step_parts.load();
         r = capture_graph(s, &s->graphs.gen[phase], &s->graphs.n_gen[phase], [&](cudaStream_t st) -> mw_status {
             mw_status q = enqueue_layers(m, R, beam, phase, st, step_parts);
@@ -2222,8 +2144,8 @@ extern "C" void mw_debug_step_parts(int parts) {
 }
 
 // ---- test entry points (include/mw_b200.h): the decode step's kernels on caller buffers, the launch path named by an argument.
-// No A/B hook changes what they run.  Shapes and the path are checked before any pointer, and all of it before anything is
-// launched, so a rejected call touches no memory.
+// Shapes and the path are checked before any pointer, and all of it before anything is launched, so a rejected call touches
+// no memory.
 extern "C" mw_status mw_step_projection_h16(const void* d_x_h16, const float* d_x_f32, const float* d_gamma, const float* d_beta,
                                             const void* d_w, const float* d_bias, const float* d_resid, void* d_out, int R, int N,
                                             int K, int flags, int path, void* stream) {
@@ -2287,10 +2209,12 @@ extern "C" mw_status mw_step_self_attention_h16(const void* d_qkv, void* d_k_cac
     DecCtl* ctl = nullptr;
     MW_CUDA_CHECK(cudaMalloc((void**)&ctl, sizeof(DecCtl)));
     cudaError_t e = cudaMemcpyAsync(ctl, &h_ctl, sizeof(DecCtl), cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess)
-        e = launch_chained(decode_attn_kernel<true>, dim3(n_heads, R), dim3(128), ctx * sizeof(float), st, qkv, 3 * d,
-                           (mw_h*)d_k_cache, (mw_h*)d_v_cache, (int64_t)d, (int64_t)ctx, (const int*)d_idx, ctx, (const DecCtl*)ctl, 0,
-                           1, qkv + d, qkv + 2 * d, 3 * d, (mw_h*)d_out, d, 0);
+    if (e == cudaSuccess) {
+        decode_attn_kernel<true><<<dim3(n_heads, R), 128, ctx * sizeof(float), st>>>(qkv, 3 * d, (mw_h*)d_k_cache, (mw_h*)d_v_cache, d, ctx,
+                                                                                     (const int*)d_idx, ctx, ctl, 0, 1, qkv + d, qkv + 2 * d,
+                                                                                     3 * d, (mw_h*)d_out, d, 0);
+        e = cudaGetLastError();
+    }
     if (e == cudaSuccess) { count_launch(); e = cudaStreamSynchronize(st); }      // h_ctl is read by the copy until then
     cudaFree(ctl);
     if (e != cudaSuccess) { set_error("mw_step_self_attention_h16: %s", cudaGetErrorString(e)); return MW_ERR_CUDA; }
@@ -2325,12 +2249,8 @@ extern "C" mw_status mw_step_cross_attention_h16(const void* d_q, const void* d_
     const mw_h* kv = (const mw_h*)d_kv;
     mw_h* out = (mw_h*)d_out;
     if (G == 1) {
-        if (unr == 8)
-            launch_chained(cross_attn_stream_kernel<8>, dim3(n_heads, B), dim3(128), 0, st, q, d, kv, kv + d, (int64_t)(2 * d), T, out, d,
-                           (const char*)nullptr, 0);
-        else
-            launch_chained(cross_attn_stream_kernel<4>, dim3(n_heads, B), dim3(128), 0, st, q, d, kv, kv + d, (int64_t)(2 * d), T, out, d,
-                           (const char*)nullptr, 0);
+        if (unr == 8) cross_attn_stream_kernel<8><<<dim3(n_heads, B), 128, 0, st>>>(q, d, kv, kv + d, 2 * d, T, out, d, nullptr, 0);
+        else cross_attn_stream_kernel<4><<<dim3(n_heads, B), 128, 0, st>>>(q, d, kv, kv + d, 2 * d, T, out, d, nullptr, 0);
         MW_LAUNCH_CHECK();
         return MW_OK;
     }

@@ -17,8 +17,6 @@ __global__ void __launch_bounds__(256)
 layernorm_kernel(const float* x /* MODE 3 writes it back: no __restrict__ */, const float* __restrict__ gamma,
                  const float* __restrict__ beta, void* out_v, int rows, int d) {
     mw_h* out = reinterpret_cast<mw_h*>(out_v);
-    pdl_trigger();
-    pdl_wait();
     const int row = blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (row >= rows) return;
@@ -119,10 +117,9 @@ mw_status layernorm_launch(const float* x, const float* gamma, const float* beta
     MW_REQUIRE(d % 128 == 0 && d >= 128 && d <= 2048, "layernorm: d=%d must be a multiple of 128 in [128, 2048]", d);
     if (rows <= 0) return MW_OK;
     const int grid = ceil_div(rows, 8);
-    // launched as a link of a dependent-launch chain (a no-op outside the decoder's step, where the neighbours are ordinary launches)
-    if (d <= 512) launch_chained(layernorm_kernel<4, 0>, dim3(grid), dim3(256), 0, st, x, gamma, beta, out_bf16, rows, d);
-    else if (d <= 1280) launch_chained(layernorm_kernel<10, 0>, dim3(grid), dim3(256), 0, st, x, gamma, beta, out_bf16, rows, d);
-    else launch_chained(layernorm_kernel<16, 0>, dim3(grid), dim3(256), 0, st, x, gamma, beta, out_bf16, rows, d);
+    if (d <= 512) layernorm_kernel<4, 0><<<grid, 256, 0, st>>>(x, gamma, beta, out_bf16, rows, d);
+    else if (d <= 1280) layernorm_kernel<10, 0><<<grid, 256, 0, st>>>(x, gamma, beta, out_bf16, rows, d);
+    else layernorm_kernel<16, 0><<<grid, 256, 0, st>>>(x, gamma, beta, out_bf16, rows, d);
     MW_LAUNCH_CHECK();
     return MW_OK;
 }

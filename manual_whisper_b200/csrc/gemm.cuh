@@ -39,10 +39,9 @@ mw_status encode_tensor_map(CUtensorMap* map, const void* base, int rank, const 
 int device_sm_count();
 
 // decode_gemm.cu: out[R, N] = X[R, K] . W[N, K]^T (+bias) (gelu: flags & 1) (+resid f32, ld = ldo) -> h16 or f32 (flags & 2),
-// R <= 256 rows, every weight byte streamed once (swap-AB tcgen05 tiles, split-K over a thread-block cluster);
-// hooks = false ignores the MW_DG_KS A/B hook (the split-K factor is then always the tuned one)
+// R <= 256 rows, every weight byte streamed once (swap-AB tcgen05 tiles, split-K over a thread-block cluster)
 bool decode_gemm_supported(int ldx, int ldw, int R, int N, int K);
 mw_status decode_gemm_launch(const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
-                             int ldo, int R, int N, int K, int flags, cudaStream_t st, bool hooks = true);
+                             int ldo, int R, int N, int K, int flags, cudaStream_t st);
 
 }  // namespace mw

@@ -59,38 +59,6 @@ inline void count_launch(int n = 1) {
     else g_launches.fetch_add((uint64_t)n, std::memory_order_relaxed);
 }
 
-// Programmatic dependent launch (the decode step is a chain of ~350 short dependent kernels): a kernel launched through
-// launch_chained() may be scheduled while its predecessor in the stream is still running.  It calls pdl_trigger() first (its
-// own successor may be scheduled as well) and pdl_wait() before it touches anything an earlier kernel of the chain writes -
-// pdl_wait() returns when the predecessor grid has completed and flushed, which transitively covers everything before it.
-// Whatever precedes pdl_wait() may only READ data that is constant during the chain (weights, encoder K/V) and write
-// nothing.  Both instructions are no-ops in a kernel launched the ordinary way.
-// OFF by default (MW_PDL=1 turns the attribute on): inside the step's CUDA graph it measured 3.84 vs 4.05 us per node on a
-// chain of stand-alone LayerNorms, but the real single-stream step got 4 % SLOWER (4.06 vs 3.89 ms) and eight concurrent
-// batches did not move - graph edges between kernel nodes are already cheap, and the early CTAs only take SM slots.
-#if defined(__CUDACC__)
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-#endif
-inline bool pdl_enabled() {
-    static const bool on = [] { const char* e = getenv("MW_PDL"); return e && e[0] == '1'; }();
-    return on;
-}
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_chained(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-
 struct DeviceGuard {
     int prev = -1;
     explicit DeviceGuard(int dev) {

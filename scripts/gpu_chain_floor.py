@@ -1,5 +1,5 @@
 """Per-node cost of a serial chain of short kernels inside a CUDA graph (what bounds the single-stream decode step):
-N dependent LayerNorm launches (rows x 1280) captured into one graph and replayed.  env MW_PDL=0/1 (dependent-launch attribute)."""
+N dependent LayerNorm launches (rows x 1280) captured into one graph and replayed."""
 import ctypes as C, json, os, sys
 import torch
 sys.path.insert(0, os.environ.get("GRAFT_REPO_ROOT", "/root/repo"))
@@ -26,4 +26,4 @@ for rows in (1, 8, 32, 160):
         for _ in range(5): gr.replay()
         e1.record(); torch.cuda.synchronize()
         out[f"rows{rows}_us_per_node"] = round(e0.elapsed_time(e1) / 5 / N * 1e3, 3)
-print(json.dumps({"pdl": os.environ.get("MW_PDL", "1"), **out}))
+print(json.dumps(out))

@@ -29,4 +29,4 @@ for name, (N, K) in shapes.items():
         out.append({"gemm": name, "N": N, "K": K, "R": R, "us": round(us, 2), "weight_GBps": round(N * K * 2 / us / 1e3, 1),
                     "TFLOPs": round(2.0 * R * N * K / us / 1e6, 1)})
         print(out[-1], file=sys.stderr, flush=True)
-print(json.dumps({"env_MW_DG_KS": os.environ.get("MW_DG_KS"), "rows": out}))
+print(json.dumps({"rows": out}))

@@ -18,11 +18,8 @@ for (N, K) in ((1280, 1280), (1280, 5120), (5120, 1280)):
             _lib.check(lib.mw_decode_gemm_h16(x.data_ptr(), w[i % 4].data_ptr(), bias.data_ptr(), None, o.data_ptr(), R, N, K, 0, st), "dg")
             torch.cuda.synchronize()
             t = stamps.cpu().numpy()
-            if os.environ.get("MW_DG_KS") == "1":
-                t[3] = t[4] = t[5] = t[2]
             d = [int(t[j + 1] - t[j]) for j in range(7)]
             if i >= 2:
                 acc = d if acc is None else [a + b for a, b in zip(acc, d)]
-        print(json.dumps({"N": N, "K": K, "R": R, "ks": os.environ.get("MW_DG_KS", "auto"),
-                          "ns": {n: round(a / 4) for n, a in zip(names, acc)}, "total_ns": round(sum(acc) / 4)}))
+        print(json.dumps({"N": N, "K": K, "R": R, "ns": {n: round(a / 4) for n, a in zip(names, acc)}, "total_ns": round(sum(acc) / 4)}))
 lib.mw_decode_gemm_debug(None)

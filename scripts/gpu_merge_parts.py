@@ -1,7 +1,7 @@
 """Decode-step anatomy with MERGED device batches: S replicas (shared weights, one stream + host thread each) of ROWS rows
 replay one kernel class of the step concurrently.  Reports ms per step and ms per 32-window batch-step equivalent.
-args: ROWS S [iters] [classes]   env MW_DG_MIN_ROWS=1000 switches the tcgen05 decode GEMM off (mma.sync kernels)."""
-import sys, json, threading, os
+args: ROWS S [iters] [classes]"""
+import sys, json, threading
 import torch
 sys.path.insert(0, ".")
 import manual_whisper_b200 as mw
@@ -13,7 +13,7 @@ only = sys.argv[4].split(",") if len(sys.argv) > 4 else None
 dev = torch.device("cuda:0"); dims = model_dims(MODEL)
 pipe = mw.load_model(MODEL, "cuda", compute_type="float16", language="zh", asr_options={"beam_size": 1},
                      vad_model=mw.InjectedVad([]), model=device_weights(dims, dev, seed=1234), max_batch=ROWS, streams_per_device=S)
-res = {"rows": ROWS, "dg_min_rows": os.environ.get("MW_DG_MIN_ROWS", "default")}
+res = {"rows": ROWS}
 for parts, name in [(4, "gemm"), (16, "cross"), (2, "ln"), (8, "self"), (32, "logits"), (63, "layers+logits")]:
     if only and name not in only:
         continue

@@ -139,3 +139,17 @@ def test_product_never_imports_the_oracle():
             if f.endswith((".py", ".cu", ".cuh", ".h")):
                 src = open(os.path.join(dirpath, f)).read()
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", src, flags=re.M), f"{f} imports the oracle"
+
+
+def test_library_reads_only_its_debug_switches_from_the_environment():
+    """The decode step has one routing, chosen from the shapes and mw_set_solo; it launches every kernel the ordinary way."""
+    csrc = os.path.join(ROOT, "manual_whisper_b200", "csrc")
+    names, dependent_launch = set(), []
+    for dirpath, _, files in os.walk(csrc):
+        for f in files:
+            src = open(os.path.join(dirpath, f)).read()
+            names |= set(re.findall(r"getenv\(\s*\"(MW_\w+)\"", src))
+            if "griddepcontrol" in src:
+                dependent_launch.append(f)
+    assert names == {"MW_STEPWISE_PREFILL", "MW_RESAMPLE_DIRECT", "MW_W2V_STOP"}
+    assert not dependent_launch

@@ -66,20 +66,9 @@ __host__ __device__ constexpr DgLayout dg_layout(int R) {
     return l;
 }
 
-__device__ __forceinline__ float dg_gelu(float v) {     // exact-erf GELU, A&S 7.1.26 (|err| < 1.5e-7), as gemm.cu
-    const float x = fabsf(v) * 0.70710678118654752f;
-    const float t = __fdividef(1.0f, fmaf(0.3275911f, x, 1.0f));
-    float p = fmaf(1.061405429f, t, -1.453152027f);
-    p = fmaf(p, t, 1.421413741f);
-    p = fmaf(p, t, -0.284496736f);
-    p = fmaf(p, t, 0.254829592f);
-    const float e = p * t * exp2f(-1.4426950408889634f * x * x);
-    return 0.5f * v * (1.0f + copysignf(1.0f - e, v));
-}
-
 __device__ __forceinline__ float dg_finish(const DgParams& p, int64_t oi, float v, float bias) {
     v += bias;
-    if (p.flags & DG_FLAG_GELU) v = dg_gelu(v);
+    if (p.flags & DG_FLAG_GELU) v = gelu_as7126(v);
     if (p.resid) v += p.resid[oi];
     return v;
 }

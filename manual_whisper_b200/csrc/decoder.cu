@@ -82,7 +82,7 @@ struct DecoderState {
     cudaEvent_t ev[2] = {nullptr, nullptr};
     // step graphs are specific to (rows, beam): a small cache keeps the last few shapes (full batches and the short
     // last batch of a recording alternate) so they are not re-captured on every call
-    bool solo = false;                   // mw_set_solo: this replica decodes alone on its GPU (latency mode, see skinny_gemm_ln)
+    bool solo = false;                   // mw_set_solo: this replica decodes alone on its GPU (latency mode, see sk_choose)
     struct Graphs { int R = 0, beam = 0; bool solo = false; int n_prefill = 0, n_gen[2] = {0, 0}; uint64_t last_use = 0; cudaGraphExec_t prefill = nullptr, gen[2] = {nullptr, nullptr}; };
     static constexpr int GRAPH_CACHE = 4;
     Graphs graph_cache[GRAPH_CACHE];
@@ -95,8 +95,10 @@ namespace mw {
 namespace {
 
 // ------------------------------------------------------------------------------------------------
-// skinny GEMM: out[r, n] = sum_k X[r, k] W[n, k] (+bias) (gelu) (+resid);  R small, N x K streamed once
-// grid (ceil(N/16), ceil(R/32)), 256 threads: warp w owns k-blocks w, w+8, ... of 32 elements.
+// skinny GEMM: out[r, n] = sum_k X[r, k] W[n, k] (+bias) (gelu) (+resid);  R small, N x K streamed once.
+// A CTA owns 32 rows of X and WT 16-row weight tiles.  Lane (g, q) = (lane / 4, lane % 4) holds the mma.sync fragments of
+// weight rows g, g + 8 and X rows t * 8 + g (t < 4), columns q * 8 .. q * 8 + 7 of each 32-wide K block.  Every warp sums
+// its share of K, parks the sums in a shared-memory slot, and the slots are summed in order.
 // ------------------------------------------------------------------------------------------------
 constexpr int SK_FLAG_GELU = 1, SK_FLAG_F32 = 2;
 
@@ -126,6 +128,72 @@ __device__ __forceinline__ void l2_prefetch_slice(const char* pf, int pf_lines) 
         asm volatile("prefetch.global.L2 [%0];" ::"l"(pf + (int64_t)i * 128));
 }
 
+// The weight fragments of WT tiles (rows n0 + 16 wt + g and + 8, clamped to N - 1) x KB blocks from column k0 (q * 8 included)
+template <int WT, int KB>
+__device__ __forceinline__ void sk_load_w(uint4 (&alo)[WT][KB], uint4 (&ahi)[WT][KB], const mw_h* W, int ldw, int N, int n0,
+                                          int g, int k0) {
+#pragma unroll
+    for (int wt = 0; wt < WT; ++wt) {
+        const mw_h* wa = W + (int64_t)min(n0 + wt * 16 + g, N - 1) * ldw + k0;
+        const mw_h* wb = W + (int64_t)min(n0 + wt * 16 + g + 8, N - 1) * ldw + k0;
+#pragma unroll
+        for (int i = 0; i < KB; ++i) {
+            alo[wt][i] = ldg_stream(wa + i * 32);
+            ahi[wt][i] = ldg_stream(wb + i * 32);
+        }
+    }
+}
+
+// The MMAs of loaded K block i against the four X fragments x_frag(t) (rows t * 8 + g).  x_frag reads X from global memory
+// or from shared memory; it is inlined, so the choice is made at compile time.
+template <int WT, int KB, typename XFrag>
+__device__ __forceinline__ void sk_mma_block(float (&c)[WT][4][4], const uint4 (&alo)[WT][KB], const uint4 (&ahi)[WT][KB], int i,
+                                             XFrag x_frag) {
+    uint4 b[4];
+#pragma unroll
+    for (int t = 0; t < 4; ++t) b[t] = x_frag(t);
+#pragma unroll
+    for (int wt = 0; wt < WT; ++wt)
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+            mma_h16_16816(c[wt][t], alo[wt][i].x, ahi[wt][i].x, alo[wt][i].y, ahi[wt][i].y, b[t].x, b[t].y);
+            mma_h16_16816(c[wt][t], alo[wt][i].z, ahi[wt][i].z, alo[wt][i].w, ahi[wt][i].w, b[t].z, b[t].w);
+        }
+}
+
+// The accumulators into a reduction slot at their fragment positions (rows t * 8 + 2q, + 1; columns 16 wt + g, + 8)
+template <int WT>
+__device__ __forceinline__ void sk_park(float (&slot)[32][WT * 16 + 1], const float (&c)[WT][4][4], int g, int q) {
+#pragma unroll
+    for (int wt = 0; wt < WT; ++wt)
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+            slot[t * 8 + 2 * q][wt * 16 + g] = c[wt][t][0];
+            slot[t * 8 + 2 * q + 1][wt * 16 + g] = c[wt][t][1];
+            slot[t * 8 + 2 * q][wt * 16 + g + 8] = c[wt][t][2];
+            slot[t * 8 + 2 * q + 1][wt * 16 + g + 8] = c[wt][t][3];
+        }
+}
+
+// Output (r0 + rl, n0 + nl): reduction slots 0 .. NS-1 summed in order (+bias) (GELU) (+resid), stored f32 or 16-bit
+template <int NS, int LD>
+__device__ __forceinline__ void sk_output(float (*red)[32][LD], int rl, int nl, int r0, int n0, int R, int N,
+                                          const float* __restrict__ bias, const float* resid, void* out, int ldo, int flags) {
+    const int r = r0 + rl, n = n0 + nl;
+    float v = 0.0f;
+#pragma unroll
+    for (int w = 0; w < NS; ++w) v += red[w][rl][nl];
+    if (r < R && n < N) {
+        if (bias) v += __ldg(bias + n);
+        if (flags & SK_FLAG_GELU) v = gelu_erff(v);
+        const int64_t oi = (int64_t)r * ldo + n;
+        if (resid) v += resid[oi];
+        if (flags & SK_FLAG_F32) reinterpret_cast<float*>(out)[oi] = v;
+        else reinterpret_cast<mw_h*>(out)[oi] = f2h(v);
+    }
+}
+
+// Any K % 32 == 0: grid (ceil(N/16), ceil(R/32)), 256 threads; warp w owns K blocks w, w+8, ...
 __global__ void __launch_bounds__(256)
 skinny_gemm_kernel(const mw_h* __restrict__ X, int ldx, const mw_h* __restrict__ W, int ldw,
                    const float* __restrict__ bias, const float* resid, void* out, int ldo, int R, int N, int K,
@@ -139,50 +207,18 @@ skinny_gemm_kernel(const mw_h* __restrict__ X, int ldx, const mw_h* __restrict__
     const mw_h* xr[4];
 #pragma unroll
     for (int t = 0; t < 4; ++t) xr[t] = X + (int64_t)min(r0 + t * 8 + g, R - 1) * ldx + q * 8;
-    float c[4][4];
-#pragma unroll
-    for (int t = 0; t < 4; ++t)
-#pragma unroll
-        for (int i = 0; i < 4; ++i) c[t][i] = 0.0f;
+    float c[1][4][4] = {};
     const int nkb = K >> 5;
 #pragma unroll 2
     for (int kb = warp; kb < nkb; kb += 8) {
         const int k = kb << 5;
-        const uint4 alo = ldg_stream(wa + k);
-        const uint4 ahi = ldg_stream(wb + k);
-        uint4 b[4];
-#pragma unroll
-        for (int t = 0; t < 4; ++t) b[t] = __ldg(reinterpret_cast<const uint4*>(xr[t] + k));
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-            mma_h16_16816(c[t], alo.x, ahi.x, alo.y, ahi.y, b[t].x, b[t].y);
-            mma_h16_16816(c[t], alo.z, ahi.z, alo.w, ahi.w, b[t].z, b[t].w);
-        }
+        const uint4 alo[1][1] = {{ldg_stream(wa + k)}}, ahi[1][1] = {{ldg_stream(wb + k)}};
+        sk_mma_block(c, alo, ahi, 0, [&](int t) { return __ldg(reinterpret_cast<const uint4*>(xr[t] + k)); });
     }
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-        red[warp][t * 8 + 2 * q][g] = c[t][0];
-        red[warp][t * 8 + 2 * q + 1][g] = c[t][1];
-        red[warp][t * 8 + 2 * q][g + 8] = c[t][2];
-        red[warp][t * 8 + 2 * q + 1][g + 8] = c[t][3];
-    }
+    sk_park(red[warp], c, g, q);
     __syncthreads();
 #pragma unroll
-    for (int o = threadIdx.x; o < 512; o += 256) {
-        const int rl = o >> 4, nl = o & 15;
-        const int r = r0 + rl, n = n0 + nl;
-        float v = 0.0f;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) v += red[w][rl][nl];
-        if (r < R && n < N) {
-            if (bias) v += __ldg(bias + n);
-            if (flags & SK_FLAG_GELU) v = 0.5f * v * (1.0f + erff(v * 0.70710678118654752f));
-            const int64_t oi = (int64_t)r * ldo + n;
-            if (resid) v += resid[oi];
-            if (flags & SK_FLAG_F32) reinterpret_cast<float*>(out)[oi] = v;
-            else reinterpret_cast<mw_h*>(out)[oi] = f2h(v);
-        }
-    }
+    for (int o = threadIdx.x; o < 512; o += 256) sk_output<8>(red, o >> 4, o & 15, r0, n0, R, N, bias, resid, out, ldo, flags);
 }
 
 // Main version: a CTA owns 16 weight rows and the whole K; its NW warps split K into contiguous runs of KB
@@ -201,73 +237,27 @@ skinny_gemm_rows16_kernel(const mw_h* __restrict__ X, int ldx, const mw_h* __res
     const int n0 = blockIdx.x * (16 * WT), r0 = blockIdx.y * 32;
     const int k_start = warp * (KB * 32) + q * 8;
     uint4 alo[WT][KB], ahi[WT][KB];
-#pragma unroll
-    for (int wt = 0; wt < WT; ++wt) {
-        const mw_h* wa = W + (int64_t)min(n0 + wt * 16 + g, N - 1) * ldw + k_start;
-        const mw_h* wb = W + (int64_t)min(n0 + wt * 16 + g + 8, N - 1) * ldw + k_start;
-#pragma unroll
-        for (int i = 0; i < KB; ++i) {
-            alo[wt][i] = ldg_stream(wa + i * 32);
-            ahi[wt][i] = ldg_stream(wb + i * 32);
-        }
-    }
+    sk_load_w(alo, ahi, W, ldw, N, n0, g, k_start);
     // the whole weight slice is in flight before the first X load is issued
     const mw_h* xr[4];
 #pragma unroll
     for (int t = 0; t < 4; ++t) xr[t] = X + (int64_t)min(r0 + t * 8 + g, R - 1) * ldx + k_start;
-    float c[WT][4][4];
+    float c[WT][4][4] = {};
 #pragma unroll
-    for (int wt = 0; wt < WT; ++wt)
-#pragma unroll
-        for (int t = 0; t < 4; ++t)
-#pragma unroll
-            for (int i = 0; i < 4; ++i) c[wt][t][i] = 0.0f;
-#pragma unroll
-    for (int i = 0; i < KB; ++i) {
-        uint4 b[4];
-#pragma unroll
-        for (int t = 0; t < 4; ++t) b[t] = __ldg(reinterpret_cast<const uint4*>(xr[t] + i * 32));
-#pragma unroll
-        for (int wt = 0; wt < WT; ++wt)
-#pragma unroll
-            for (int t = 0; t < 4; ++t) {
-                mma_h16_16816(c[wt][t], alo[wt][i].x, ahi[wt][i].x, alo[wt][i].y, ahi[wt][i].y, b[t].x, b[t].y);
-                mma_h16_16816(c[wt][t], alo[wt][i].z, ahi[wt][i].z, alo[wt][i].w, ahi[wt][i].w, b[t].z, b[t].w);
-            }
-    }
+    for (int i = 0; i < KB; ++i)
+        sk_mma_block(c, alo, ahi, i, [&](int t) { return __ldg(reinterpret_cast<const uint4*>(xr[t] + i * 32)); });
     l2_prefetch_slice(pf, pf_lines);
-#pragma unroll
-    for (int wt = 0; wt < WT; ++wt)
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-            red[warp][t * 8 + 2 * q][wt * 16 + g] = c[wt][t][0];
-            red[warp][t * 8 + 2 * q + 1][wt * 16 + g] = c[wt][t][1];
-            red[warp][t * 8 + 2 * q][wt * 16 + g + 8] = c[wt][t][2];
-            red[warp][t * 8 + 2 * q + 1][wt * 16 + g + 8] = c[wt][t][3];
-        }
+    sk_park(red[warp], c, g, q);
     __syncthreads();
-    for (int o = threadIdx.x; o < 32 * 16 * WT; o += NW * 32) {
-        const int rl = o / (16 * WT), nl = o % (16 * WT);
-        const int r = r0 + rl, n = n0 + nl;
-        float v = 0.0f;
-#pragma unroll
-        for (int w = 0; w < NW; ++w) v += red[w][rl][nl];
-        if (r < R && n < N) {
-            if (bias) v += __ldg(bias + n);
-            if (flags & SK_FLAG_GELU) v = 0.5f * v * (1.0f + erff(v * 0.70710678118654752f));
-            const int64_t oi = (int64_t)r * ldo + n;
-            if (resid) v += resid[oi];
-            if (flags & SK_FLAG_F32) reinterpret_cast<float*>(out)[oi] = v;
-            else reinterpret_cast<mw_h*>(out)[oi] = f2h(v);
-        }
-    }
+    for (int o = threadIdx.x; o < 32 * 16 * WT; o += NW * 32)
+        sk_output<NW>(red, o / (16 * WT), o % (16 * WT), r0, n0, R, N, bias, resid, out, ldo, flags);
 }
 
 // LayerNorm folded into the projection that consumes it (QKV, cross-attention Q, fc1).  A decode step is a serial chain of
 // ~350 graph nodes and a node costs >= 3.3 us however little it does (scripts/gpu_chain_floor.py), so the 96 stand-alone
 // LayerNorm launches of a large-v3 step were 0.7 ms of a 3.9 ms single-stream step.  Here every CTA normalises its 32 rows
-// itself - warp per row, the SAME lane mapping, summation order and rounding as layernorm_kernel (elementwise.cu), so the
-// 16-bit operand is bit-identical to the stand-alone kernel's - into shared memory, and the MMAs read it from there.
+// itself - warp per row, with the ln_stats / ln_apply / pack_h16x4 of layernorm_kernel (mw_common.cuh), so the 16-bit
+// operand is bit-identical to the stand-alone kernel's - into shared memory, and the MMAs read it from there.
 // The price is L2 traffic (each CTA reads the fp32 rows instead of the 16-bit copy), not HBM traffic.
 template <int KB, int NW, int WT>
 __global__ void __launch_bounds__(NW * 32, WT == 2 ? 2 : 1)
@@ -297,109 +287,31 @@ skinny_gemm_ln_kernel(const float* __restrict__ x, const float* __restrict__ gam
         for (int h = 0; h < 2; ++h) {
             const int rl = rl0 + h * NW;
             if (rl >= 32 || r0 + rl >= R) break;      // rows past the batch: their products are never stored (warp-uniform)
-            float s = 0.0f;
+            float s = 0.0f, mean, rstd;
 #pragma unroll
-            for (int i = 0; i < MAXV; ++i) s += (v[h][i].x + v[h][i].y) + (v[h][i].z + v[h][i].w);
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-            const float mean = s / (float)K;
-            float qq = 0.0f;
-#pragma unroll
-            for (int i = 0; i < MAXV; ++i) {
-                const float a = v[h][i].x - mean, b = v[h][i].y - mean, c = v[h][i].z - mean, e = v[h][i].w - mean;
-                qq += (a * a + b * b) + (c * c + e * e);
-            }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) qq += __shfl_xor_sync(0xffffffffu, qq, o);
-            const float rstd = rsqrtf(qq / (float)K + 1e-5f);
+            for (int i = 0; i < MAXV; ++i) s += sum4(v[h][i]);
+            ln_stats(s, v[h], MAXV, K, mean, rstd);
             uint2* o2 = reinterpret_cast<uint2*>(xs + rl * XS);
 #pragma unroll
-            for (int i = 0; i < MAXV; ++i) {
-                const float4 gg = __ldg(g4 + i * 32 + lane), bb = __ldg(b4 + i * 32 + lane);
-                const float y0 = (v[h][i].x - mean) * rstd * gg.x + bb.x, y1 = (v[h][i].y - mean) * rstd * gg.y + bb.y;
-                const float y2 = (v[h][i].z - mean) * rstd * gg.z + bb.z, y3 = (v[h][i].w - mean) * rstd * gg.w + bb.w;
-                mw_h2 h0 = f2h2(y0, y1);
-                mw_h2 h1 = f2h2(y2, y3);
-                uint2 u;
-                u.x = *reinterpret_cast<uint32_t*>(&h0);
-                u.y = *reinterpret_cast<uint32_t*>(&h1);
-                o2[i * 32 + lane] = u;
-            }
+            for (int i = 0; i < MAXV; ++i)
+                o2[i * 32 + lane] = pack_h16x4(ln_apply(v[h][i], mean, rstd, __ldg(g4 + i * 32 + lane), __ldg(b4 + i * 32 + lane)));
         }
     }
     // ---- the projection, as skinny_gemm_rows16_kernel with the X fragments read from shared memory
     const int k_start = warp * (KB * 32) + q * 8;
     uint4 alo[WT][KB], ahi[WT][KB];
-#pragma unroll
-    for (int wt = 0; wt < WT; ++wt) {
-        const mw_h* wa = W + (int64_t)min(n0 + wt * 16 + g, N - 1) * ldw + k_start;
-        const mw_h* wb = W + (int64_t)min(n0 + wt * 16 + g + 8, N - 1) * ldw + k_start;
-#pragma unroll
-        for (int i = 0; i < KB; ++i) {
-            alo[wt][i] = ldg_stream(wa + i * 32);
-            ahi[wt][i] = ldg_stream(wb + i * 32);
-        }
-    }
+    sk_load_w(alo, ahi, W, ldw, N, n0, g, k_start);
     __syncthreads();
-    float c[WT][4][4];
+    float c[WT][4][4] = {};
 #pragma unroll
-    for (int wt = 0; wt < WT; ++wt)
-#pragma unroll
-        for (int t = 0; t < 4; ++t)
-#pragma unroll
-            for (int i = 0; i < 4; ++i) c[wt][t][i] = 0.0f;
-#pragma unroll
-    for (int i = 0; i < KB; ++i) {
-        uint4 b[4];
-#pragma unroll
-        for (int t = 0; t < 4; ++t) b[t] = *reinterpret_cast<const uint4*>(xs + (t * 8 + g) * XS + k_start + i * 32);
-#pragma unroll
-        for (int wt = 0; wt < WT; ++wt)
-#pragma unroll
-            for (int t = 0; t < 4; ++t) {
-                mma_h16_16816(c[wt][t], alo[wt][i].x, ahi[wt][i].x, alo[wt][i].y, ahi[wt][i].y, b[t].x, b[t].y);
-                mma_h16_16816(c[wt][t], alo[wt][i].z, ahi[wt][i].z, alo[wt][i].w, ahi[wt][i].w, b[t].z, b[t].w);
-            }
-    }
+    for (int i = 0; i < KB; ++i)
+        sk_mma_block(c, alo, ahi, i, [&](int t) { return *reinterpret_cast<const uint4*>(xs + (t * 8 + g) * XS + k_start + i * 32); });
     l2_prefetch_slice(pf, pf_lines);
     __syncthreads();          // every warp has read its X fragments: the reduction buffer may overwrite them
-#pragma unroll
-    for (int wt = 0; wt < WT; ++wt)
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-            red[warp][t * 8 + 2 * q][wt * 16 + g] = c[wt][t][0];
-            red[warp][t * 8 + 2 * q + 1][wt * 16 + g] = c[wt][t][1];
-            red[warp][t * 8 + 2 * q][wt * 16 + g + 8] = c[wt][t][2];
-            red[warp][t * 8 + 2 * q + 1][wt * 16 + g + 8] = c[wt][t][3];
-        }
+    sk_park(red[warp], c, g, q);
     __syncthreads();
-    for (int o = threadIdx.x; o < 32 * 16 * WT; o += NW * 32) {
-        const int rl = o / (16 * WT), nl = o % (16 * WT);
-        const int r = r0 + rl, n = n0 + nl;
-        float v = 0.0f;
-#pragma unroll
-        for (int w = 0; w < NW; ++w) v += red[w][rl][nl];
-        if (r < R && n < N) {
-            if (bias) v += __ldg(bias + n);
-            if (flags & SK_FLAG_GELU) v = 0.5f * v * (1.0f + erff(v * 0.70710678118654752f));
-            out[(int64_t)r * ldo + n] = f2h(v);
-        }
-    }
-}
-
-template <int KB, int NW>
-mw_status launch_ln_rows16(const float* x, const float* gamma, const float* beta, const void* W, int ldw, const float* bias,
-                           void* out, int ldo, int R, int N, int flags, cudaStream_t st, const char* pf, int pf_lines) {
-    constexpr int WT = 2, K = KB * NW * 32;
-    constexpr int xs_bytes = 32 * (K + 32) * 2, red_bytes = NW * 32 * (WT * 16 + 1) * 4;
-    constexpr int smem = xs_bytes > red_bytes ? xs_bytes : red_bytes;
-    static PerDeviceOnce attr_once;
-    MW_CUDA_CHECK(attr_once.run([&] { return cudaFuncSetAttribute(skinny_gemm_ln_kernel<KB, NW, WT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); }));
-    dim3 grid(ceil_div(N, 16 * WT), ceil_div(R, 32));
-    skinny_gemm_ln_kernel<KB, NW, WT><<<grid, NW * 32, smem, st>>>(x, gamma, beta, (const mw_h*)W, ldw, bias, (mw_h*)out, ldo, R, N,
-                                                                  flags, pf, pf_lines);
-    MW_LAUNCH_CHECK();
-    return MW_OK;
+    for (int o = threadIdx.x; o < 32 * 16 * WT; o += NW * 32)         // 16-bit output, no residual
+        sk_output<NW>(red, o / (16 * WT), o % (16 * WT), r0, n0, R, N, bias, nullptr, out, ldo, flags & SK_FLAG_GELU);
 }
 
 // K = 5120-class shapes (16 warps): the same two-tile idea needs 160 weight registers, so K is walked in two halves of
@@ -416,42 +328,18 @@ skinny_gemm_rows32_khalf_kernel(const mw_h* __restrict__ X, int ldx, const mw_h*
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int g = lane >> 2, q = lane & 3;
     const int n0 = blockIdx.x * (16 * WT), r0 = blockIdx.y * 32;
-    float c[WT][4][4];
-#pragma unroll
-    for (int wt = 0; wt < WT; ++wt)
-#pragma unroll
-        for (int t = 0; t < 4; ++t)
-#pragma unroll
-            for (int i = 0; i < 4; ++i) c[wt][t][i] = 0.0f;
+    float c[WT][4][4] = {};
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
         const int k_start = h * (NW * KB * 32) + warp * (KB * 32) + q * 8;
         uint4 alo[WT][KB], ahi[WT][KB];
-#pragma unroll
-        for (int wt = 0; wt < WT; ++wt) {
-            const mw_h* wa = W + (int64_t)min(n0 + wt * 16 + g, N - 1) * ldw + k_start;
-            const mw_h* wb = W + (int64_t)min(n0 + wt * 16 + g + 8, N - 1) * ldw + k_start;
-#pragma unroll
-            for (int i = 0; i < KB; ++i) {
-                alo[wt][i] = ldg_stream(wa + i * 32);
-                ahi[wt][i] = ldg_stream(wb + i * 32);
-            }
-        }
+        sk_load_w(alo, ahi, W, ldw, N, n0, g, k_start);
         // this half's weights are in flight before its X loads are issued
 #pragma unroll
-        for (int i = 0; i < KB; ++i) {
-            uint4 b[4];
-#pragma unroll
-            for (int t = 0; t < 4; ++t)
-                b[t] = __ldg(reinterpret_cast<const uint4*>(X + (int64_t)min(r0 + t * 8 + g, R - 1) * ldx + k_start + i * 32));
-#pragma unroll
-            for (int wt = 0; wt < WT; ++wt)
-#pragma unroll
-                for (int t = 0; t < 4; ++t) {
-                    mma_h16_16816(c[wt][t], alo[wt][i].x, ahi[wt][i].x, alo[wt][i].y, ahi[wt][i].y, b[t].x, b[t].y);
-                    mma_h16_16816(c[wt][t], alo[wt][i].z, ahi[wt][i].z, alo[wt][i].w, ahi[wt][i].w, b[t].z, b[t].w);
-                }
-        }
+        for (int i = 0; i < KB; ++i)
+            sk_mma_block(c, alo, ahi, i, [&](int t) {
+                return __ldg(reinterpret_cast<const uint4*>(X + (int64_t)min(r0 + t * 8 + g, R - 1) * ldx + k_start + i * 32));
+            });
     }
     l2_prefetch_slice(pf, pf_lines);
     // warps 8..15 park their partial sums, warps 0..7 fold them in (same fragment positions), then the usual 8-slot reduce
@@ -471,124 +359,152 @@ skinny_gemm_rows32_khalf_kernel(const mw_h* __restrict__ X, int ldx, const mw_h*
         }
         __syncthreads();
     }
-    for (int o = threadIdx.x; o < 32 * 16 * WT; o += NW * 32) {
-        const int rl = o / (16 * WT), nl = o % (16 * WT);
-        const int r = r0 + rl, n = n0 + nl;
-        float v = 0.0f;
-#pragma unroll
-        for (int w = 0; w < NW / 2; ++w) v += red[w][rl][nl];
-        if (r < R && n < N) {
-            if (bias) v += __ldg(bias + n);
-            if (flags & SK_FLAG_GELU) v = 0.5f * v * (1.0f + erff(v * 0.70710678118654752f));
-            const int64_t oi = (int64_t)r * ldo + n;
-            if (resid) v += resid[oi];
-            if (flags & SK_FLAG_F32) reinterpret_cast<float*>(out)[oi] = v;
-            else reinterpret_cast<mw_h*>(out)[oi] = f2h(v);
-        }
-    }
+    for (int o = threadIdx.x; o < 32 * 16 * WT; o += NW * 32)
+        sk_output<NW / 2>(red, o / (16 * WT), o % (16 * WT), r0, n0, R, N, bias, resid, out, ldo, flags);
 }
 
-// Which kernel a decode-step projection runs.  SK_ROUTE is the step's own routing; the others force one kernel
-// (mw_step_projection_h16).
-enum SkPath { SK_ROUTE, SK_ROWS16_WT1, SK_ROWS16_WT2, SK_KHALF_WT1, SK_KHALF_WT2, SK_GENERIC, SK_LN_FUSED, SK_LN_SEPARATE };
+// The tuned shapes (KB, NW) of the mma.sync kernels, K = KB * NW * 32 (the d_model and ffn widths of the Whisper sizes and
+// the test dims): rows16 with one weight tile serves all of them; the K-halved kernel replaces it where sk_k_halved holds,
+// and where sk_two_tiles holds rows16 and the fused LayerNorm projection run with two tiles.  Other K: the generic kernel.
+#define MW_SK(X)                                \
+    X(5, 8)     /* 1280  (large) */             \
+    X(10, 16)   /* 5120  (large ffn) */         \
+    X(4, 8)     /* 1024  (medium) */            \
+    X(8, 16)    /* 4096  (medium ffn) */        \
+    X(3, 8)     /* 768   (small) */             \
+    X(6, 16)    /* 3072  (small ffn) */         \
+    X(2, 8)     /* 512   (base / test ffn) */   \
+    X(4, 16)    /* 2048  (base ffn) */          \
+    X(3, 4)     /* 384   (tiny) */              \
+    X(6, 8)     /* 1536  (tiny ffn) */          \
+    X(1, 4)     /* 128   (test dims) */         \
+    X(1, 8)     /* 256 */
 
-// rows from which the tcgen05 decode GEMM takes over the projections the step routes to it (see skinny_gemm)
+// two weight tiles fit the registers
+constexpr bool sk_two_tiles(int KB, int NW) { return NW <= 8 && KB <= 5; }
+// the 16-warp shapes, as two halves of KB / 2 blocks per warp
+constexpr bool sk_k_halved(int KB, int NW) { return NW == 16 && KB % 2 == 0 && KB / 2 <= 5; }
+
+// warps per CTA of the tuned entry for K, 0 when K has none
+int sk_table_warps(int K) {
+#define MW_SK_WARPS(kb, nw) if (K == kb * nw * 32) return nw;
+    MW_SK(MW_SK_WARPS)
+#undef MW_SK_WARPS
+    return 0;
+}
+
+// The kernels of a decode-step projection.  A caller asks for SK_ROUTE (the step's own routing) or forces one kernel
+// (mw_step_projection_h16); sk_choose answers with the kernel that runs, or SK_NONE.
+enum SkKernel { SK_ROUTE, SK_ROWS16_WT1, SK_ROWS16_WT2, SK_KHALF_WT1, SK_KHALF_WT2, SK_GENERIC, SK_LN_FUSED, SK_DECODE_GEMM, SK_NONE };
+const char* const SK_NAME[SK_NONE] = {"routed", "rows16", "two-tile rows16", "K-halved", "K-halved", "generic",
+                                      "fused LayerNorm (16-bit output)", "decode GEMM"};
+
+// rows from which the tcgen05 decode GEMM takes over the projections the step routes to it
 constexpr int DG_MIN_ROWS = 96;
 
-// The tuned projections of skinny_gemm (its MW_SK table): warps per CTA for K = KB * NW * 32, 0 when K has no entry.
-// The K-halved kernel serves the 16-warp entries; two weight tiles fit the registers for KB <= 5 with at most 8 warps.
-int sk_table_warps(int K) {
-    switch (K) {
-        case 128: case 384: return 4;
-        case 256: case 512: case 768: case 1024: case 1280: case 1536: return 8;
-        case 2048: case 3072: case 4096: case 5120: return 16;
-        default: return 0;
+// The kernel for out[R, N] = X[R, K] W[N, K]^T (row pitches ldx, ldw) as `path` asks, X = LayerNorm(x) when `ln`; SK_NONE
+// when a forced kernel does not exist for K (or, SK_LN_FUSED, for fp32 output).  The step's routing:
+//  * R >= DG_MIN_ROWS rows (merged greedy batches): the weight-stationary tcgen05 kernel (decode_gemm.cu) streams W once
+//    for all rows; the mma.sync kernels re-read it per 32-row block (from L2 after the first block) and stay in charge of
+//    the 32-row batches they were tuned on and of beam search, where they measured faster (DESIGN.md section 4: a decode
+//    step is a chain of ~360 latency-bound launches, so bytes saved do not buy time unless the launch is also shorter).
+//    The step passes allow_dg = (beam <= 1) for the layer projections; the vocabulary projection (enqueue_logits) keeps
+//    it, so at R >= 96 rows it runs on the decode GEMM in beam search as well.
+//  * LayerNorm: with `solo` (mw_set_solo: the replica decodes alone on its GPU) ONE launch where the fused kernel applies
+//    (16-bit output, two tiles, rows that do not go to the decode GEMM).  Otherwise the stand-alone LayerNorm, then the
+//    projection as routed without `solo`.  Both give the same bits; which is faster depends on what else the GPU is doing -
+//    measured on large-v3, ms per 32-row step, fused / separate: one batch in flight 3.71 / 3.88 (96 graph nodes fewer),
+//    two 2.78 / 2.75, four 2.33 / 2.20, eight 2.30 / 2.09.  With several batches in flight a node's fixed cost is hidden by
+//    the other batches anyway, and every CTA now holds its SM slot (and 84 KB of shared memory) for the ~1 us it spends
+//    normalising 32 rows before it asks for its weights.  (It is not the extra L2->SM traffic: reading the 16-bit operand
+//    twice in the plain kernels costs nothing at eight streams.)
+//  * the K-halved kernel with one weight tile for a lone batch (3.87 -> 3.76 ms per single-stream step), else two; two-tile
+//    rows16 where it fits, else one tile; the generic kernel for K outside MW_SK.
+SkKernel sk_choose(int ldx, int ldw, int R, int N, int K, int flags, SkKernel path, bool allow_dg, bool solo, bool ln) {
+    const bool to_dg = allow_dg && R >= DG_MIN_ROWS && decode_gemm_supported(ldx, ldw, R, N, K);
+    const int nw = sk_table_warps(K), kb = nw ? K / (nw * 32) : 0;
+    const bool two_tiles = nw && sk_two_tiles(kb, nw), k_halved = nw && sk_k_halved(kb, nw);
+    if (ln && (path == SK_LN_FUSED || (path == SK_ROUTE && solo && !to_dg)) && two_tiles && !(flags & SK_FLAG_F32))
+        return SK_LN_FUSED;
+    if (ln) solo = false;
+    switch (path) {
+        case SK_ROUTE:
+            if (to_dg) return SK_DECODE_GEMM;
+            if (k_halved) return solo ? SK_KHALF_WT1 : SK_KHALF_WT2;
+            return two_tiles ? SK_ROWS16_WT2 : nw ? SK_ROWS16_WT1 : SK_GENERIC;
+        case SK_GENERIC: return path;
+        case SK_ROWS16_WT1: return nw ? path : SK_NONE;
+        case SK_ROWS16_WT2: return two_tiles ? path : SK_NONE;
+        case SK_KHALF_WT1: case SK_KHALF_WT2: return k_halved ? path : SK_NONE;
+        default: return SK_NONE;
     }
 }
-bool sk_has_rows16_wt2(int K) { const int nw = sk_table_warps(K); return nw && nw <= 8 && K / (nw * 32) <= 5; }
-bool sk_has_khalf(int K) { const int nw = sk_table_warps(K); return nw == 16 && (K / (nw * 32)) % 2 == 0 && K / (nw * 32) / 2 <= 5; }
-bool sk_has_ln_fused(int K) { return sk_has_rows16_wt2(K); }    // the MW_SKLN table of skinny_gemm_ln
 
+mw_status sk_missing(const char* who, SkKernel path, int K) {
+    set_error("%s: no %s kernel for K=%d", who, SK_NAME[path], K);
+    return MW_ERR_UNSUPPORTED;
+}
+
+// kernel k of a tuned shape; x, gamma, beta: the fp32 rows and the LayerNorm of SK_LN_FUSED
 template <int KB, int NW>
-mw_status launch_rows16(const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
-                        int ldo, int R, int N, int K, int flags, cudaStream_t st, const char* pf, int pf_lines, bool solo,
-                        SkPath path) {
-    constexpr int WT = (NW <= 8 && KB <= 5) ? 2 : 1;          // two weight tiles where the registers allow it
-    const bool routed = path == SK_ROUTE;
-    if ((path == SK_KHALF_WT1 || path == SK_KHALF_WT2) && !(NW == 16 && KB % 2 == 0 && KB / 2 <= 5)) {
-        set_error("skinny gemm: no K-halved kernel for K=%d", K);
-        return MW_ERR_UNSUPPORTED;
-    }
-    if (path == SK_ROWS16_WT2 && WT != 2) {
-        set_error("skinny gemm: no two-tile rows16 kernel for K=%d", K);
-        return MW_ERR_UNSUPPORTED;
-    }
-    if constexpr (NW == 16 && KB % 2 == 0 && KB / 2 <= 5) {
-        if (routed || path == SK_KHALF_WT1 || path == SK_KHALF_WT2) {
-            const bool one = routed ? solo : path == SK_KHALF_WT1;
-            if (one) {       // a lone batch: 3.87 -> 3.76 ms per single-stream step
-                dim3 grid(ceil_div(N, 16), ceil_div(R, 32));
-                skinny_gemm_rows32_khalf_kernel<KB / 2, NW, 1><<<grid, NW * 32, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias,
-                                                                                        resid, out, ldo, R, N, K, flags, pf, pf_lines);
-            } else {
-                dim3 grid(ceil_div(N, 32), ceil_div(R, 32));
-                skinny_gemm_rows32_khalf_kernel<KB / 2, NW, 2><<<grid, NW * 32, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias,
-                                                                                        resid, out, ldo, R, N, K, flags, pf, pf_lines);
-            }
-            MW_LAUNCH_CHECK();
-            return MW_OK;
+mw_status launch_tuned(SkKernel k, const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
+                       int ldo, int R, int N, int K, int flags, cudaStream_t st, const char* pf, int pf_lines, const float* x,
+                       const float* gamma, const float* beta) {
+    const dim3 grid(ceil_div(N, k == SK_ROWS16_WT1 || k == SK_KHALF_WT1 ? 16 : 32), ceil_div(R, 32)), block(NW * 32);
+    const mw_h* Xh = (const mw_h*)X;
+    const mw_h* Wh = (const mw_h*)W;
+    if (k == SK_ROWS16_WT1)
+        skinny_gemm_rows16_kernel<KB, NW, 1><<<grid, block, 0, st>>>(Xh, ldx, Wh, ldw, bias, resid, out, ldo, R, N, K, flags, pf, pf_lines);
+    if constexpr (sk_two_tiles(KB, NW)) {
+        if (k == SK_ROWS16_WT2)
+            skinny_gemm_rows16_kernel<KB, NW, 2><<<grid, block, 0, st>>>(Xh, ldx, Wh, ldw, bias, resid, out, ldo, R, N, K, flags, pf,
+                                                                        pf_lines);
+        if (k == SK_LN_FUSED) {
+            constexpr int xs_bytes = 32 * (KB * NW * 32 + 32) * 2, red_bytes = NW * 32 * (2 * 16 + 1) * 4;
+            constexpr int smem = xs_bytes > red_bytes ? xs_bytes : red_bytes;
+            static PerDeviceOnce attr_once;
+            MW_CUDA_CHECK(attr_once.run([&] { return cudaFuncSetAttribute(skinny_gemm_ln_kernel<KB, NW, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); }));
+            skinny_gemm_ln_kernel<KB, NW, 2><<<grid, block, smem, st>>>(x, gamma, beta, Wh, ldw, bias, (mw_h*)out, ldo, R, N, flags, pf,
+                                                                       pf_lines);
         }
     }
-    if (WT == 2 && (routed || path == SK_ROWS16_WT2)) {
-        dim3 grid(ceil_div(N, 32), ceil_div(R, 32));
-        skinny_gemm_rows16_kernel<KB, NW, WT><<<grid, NW * 32, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias, resid, out, ldo,
-                                                                       R, N, K, flags, pf, pf_lines);
-    } else {
-        dim3 grid(ceil_div(N, 16), ceil_div(R, 32));
-        skinny_gemm_rows16_kernel<KB, NW, 1><<<grid, NW * 32, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias, resid, out, ldo,
-                                                                      R, N, K, flags, pf, pf_lines);
+    if constexpr (sk_k_halved(KB, NW)) {
+        if (k == SK_KHALF_WT1)
+            skinny_gemm_rows32_khalf_kernel<KB / 2, NW, 1><<<grid, block, 0, st>>>(Xh, ldx, Wh, ldw, bias, resid, out, ldo, R, N, K, flags,
+                                                                                  pf, pf_lines);
+        if (k == SK_KHALF_WT2)
+            skinny_gemm_rows32_khalf_kernel<KB / 2, NW, 2><<<grid, block, 0, st>>>(Xh, ldx, Wh, ldw, bias, resid, out, ldo, R, N, K, flags,
+                                                                                  pf, pf_lines);
     }
     MW_LAUNCH_CHECK();
     return MW_OK;
 }
 
-// `next_w` / `next_bytes`: the weight matrix of the projection that follows this one in the step (prefetched into L2)
-mw_status skinny_gemm(const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
-                      int ldo, int R, int N, int K, int flags, cudaStream_t st, bool allow_dg = true,
-                      const void* next_w = nullptr, int64_t next_bytes = 0, bool solo = false, SkPath path = SK_ROUTE) {
-    const bool routed = path == SK_ROUTE;
+// kernel k of sk_choose.  `next_w` / `next_bytes`: the weight matrix of the projection that follows this one in the step
+// (prefetched into L2)
+mw_status sk_launch(SkKernel k, const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
+                    int ldo, int R, int N, int K, int flags, cudaStream_t st, const void* next_w, int64_t next_bytes,
+                    const float* x = nullptr, const float* gamma = nullptr, const float* beta = nullptr) {
+    if (k == SK_DECODE_GEMM) return decode_gemm_launch(X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st);
     const char* pf = (const char*)next_w;
     const int pf_lines = pf ? (int)(next_bytes / 128) : 0;
-    // R >= DG_MIN_ROWS rows (merged greedy batches): the weight-stationary tcgen05 kernel (decode_gemm.cu) streams W once
-    // for all rows; the mma.sync kernels below re-read it per 32-row block (from L2 after the first block) and stay in charge
-    // of the 32-row batches they were tuned on and of beam search, where they measured faster (DESIGN.md section 4: a decode
-    // step is a chain of ~360 latency-bound launches, so bytes saved do not buy time unless the launch is also shorter).
-    // The step passes allow_dg = (beam <= 1) for the layer projections; the vocabulary projection (enqueue_logits) keeps the
-    // default, so at R >= 96 rows it runs on the decode GEMM in beam search as well.
-    if (routed && allow_dg && R >= DG_MIN_ROWS && decode_gemm_supported(ldx, ldw, R, N, K))
-        return decode_gemm_launch(X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st);
-    if (!routed && path != SK_GENERIC && !sk_table_warps(K)) {
-        set_error("skinny gemm: no tuned kernel for K=%d (the generic kernel serves it)", K);
-        return MW_ERR_UNSUPPORTED;
-    }
-#define MW_SK(kb, nw) if (path != SK_GENERIC && K == kb * nw * 32) return launch_rows16<kb, nw>(X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st, pf, pf_lines, solo, path)
-    MW_SK(5, 8);    // 1280  (large)
-    MW_SK(10, 16);  // 5120  (large ffn)
-    MW_SK(4, 8);    // 1024  (medium)
-    MW_SK(8, 16);   // 4096  (medium ffn)
-    MW_SK(3, 8);    // 768   (small)
-    MW_SK(6, 16);   // 3072  (small ffn)
-    MW_SK(2, 8);    // 512   (base / test ffn)
-    MW_SK(4, 16);   // 2048  (base ffn)
-    MW_SK(3, 4);    // 384   (tiny)
-    MW_SK(6, 8);    // 1536  (tiny ffn)
-    MW_SK(1, 4);    // 128   (test dims)
-    MW_SK(1, 8);    // 256
-#undef MW_SK
+#define MW_SK_LAUNCH(kb, nw) \
+    if (k != SK_GENERIC && K == kb * nw * 32) \
+        return launch_tuned<kb, nw>(k, X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st, pf, pf_lines, x, gamma, beta);
+    MW_SK(MW_SK_LAUNCH)
+#undef MW_SK_LAUNCH
     dim3 grid(ceil_div(N, 16), ceil_div(R, 32));
     skinny_gemm_kernel<<<grid, 256, 0, st>>>((const mw_h*)X, ldx, (const mw_h*)W, ldw, bias, resid, out, ldo, R, N, K, flags);
     MW_LAUNCH_CHECK();
     return MW_OK;
+}
+
+mw_status skinny_gemm(const void* X, int ldx, const void* W, int ldw, const float* bias, const float* resid, void* out,
+                      int ldo, int R, int N, int K, int flags, cudaStream_t st, bool allow_dg = true,
+                      const void* next_w = nullptr, int64_t next_bytes = 0, bool solo = false, SkKernel path = SK_ROUTE) {
+    const SkKernel k = sk_choose(ldx, ldw, R, N, K, flags, path, allow_dg, solo, false);
+    if (k == SK_NONE) return sk_missing("skinny gemm", path, K);
+    return sk_launch(k, X, ldx, W, ldw, bias, resid, out, ldo, R, N, K, flags, st, next_w, next_bytes);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -601,39 +517,17 @@ __global__ void embed_kernel(const int* __restrict__ cur_tok, const mw_h* __rest
         x[(int64_t)r * d + i] = h2f(emb[(int64_t)tok * d + i]) + pos_emb[(int64_t)pos * d + i];
 }
 
-// LayerNorm + projection.  `solo` (mw_set_solo: the replica decodes alone on its GPU): ONE launch where the fused kernel
-// applies (16-bit output, no residual, K = d_model of a supported size, rows that do not go to the tcgen05 decode GEMM).
-// Otherwise the stand-alone LayerNorm into `ln_buf` and skinny_gemm.  Both give the same bits; which is faster depends on
-// what else the GPU is doing - measured on large-v3, ms per 32-row step, fused / separate: one batch in flight 3.71 / 3.88
-// (96 graph nodes fewer), two 2.78 / 2.75, four 2.33 / 2.20, eight 2.30 / 2.09.  With several batches in flight a node's
-// fixed cost is hidden by the other batches anyway, and every CTA now holds its SM slot (and 84 KB of shared memory) for the
-// ~1 us it spends normalising 32 rows before it asks for its weights.  (It is not the extra L2->SM traffic: reading the
-// 16-bit operand twice in the plain kernels costs nothing at eight streams.)
+// LayerNorm + projection (the routing: sk_choose): the fused kernel, or the stand-alone LayerNorm into `ln_buf` and the projection
 mw_status skinny_gemm_ln(const float* x, const float* gamma, const float* beta, void* ln_buf, const void* W, const float* bias,
                          void* out, int ldo, int R, int N, int K, int flags, cudaStream_t st, bool allow_dg, const void* next_w,
-                         int64_t next_bytes, bool solo, SkPath path = SK_ROUTE) {
-    const bool fuse = path == SK_LN_FUSED || (path == SK_ROUTE && solo);
-    const bool to_dg = path != SK_LN_FUSED && allow_dg && R >= DG_MIN_ROWS && decode_gemm_supported(K, K, R, N, K);
-    if (path == SK_LN_FUSED && (!sk_has_ln_fused(K) || (flags & SK_FLAG_F32))) {
-        set_error("skinny gemm: no fused LayerNorm projection for K=%d%s", K, (flags & SK_FLAG_F32) ? " with fp32 output" : "");
-        return MW_ERR_UNSUPPORTED;
+                         int64_t next_bytes, bool solo, SkKernel path = SK_ROUTE) {
+    const SkKernel k = sk_choose(K, K, R, N, K, flags, path, allow_dg, solo, true);
+    if (k == SK_NONE) return sk_missing("skinny gemm", path, K);
+    if (k != SK_LN_FUSED) {
+        mw_status r = layernorm_launch(x, gamma, beta, ln_buf, R, K, st);
+        if (r != MW_OK) return r;
     }
-    if (fuse && !to_dg && !(flags & SK_FLAG_F32)) {
-        const char* pf = (const char*)next_w;
-        const int pf_lines = pf ? (int)(next_bytes / 128) : 0;
-#define MW_SKLN(kb, nw) if (K == kb * nw * 32) return launch_ln_rows16<kb, nw>(x, gamma, beta, W, K, bias, out, ldo, R, N, flags, st, pf, pf_lines)
-        MW_SKLN(5, 8);    // 1280  (large)
-        MW_SKLN(4, 8);    // 1024  (medium)
-        MW_SKLN(3, 8);    // 768   (small)
-        MW_SKLN(2, 8);    // 512   (base)
-        MW_SKLN(3, 4);    // 384   (tiny)
-        MW_SKLN(1, 4);    // 128   (test dims)
-        MW_SKLN(1, 8);    // 256
-#undef MW_SKLN
-    }
-    mw_status r = layernorm_launch(x, gamma, beta, ln_buf, R, K, st);
-    if (r != MW_OK) return r;
-    return skinny_gemm(ln_buf, K, W, K, bias, nullptr, out, ldo, R, N, K, flags, st, allow_dg, next_w, next_bytes, false, SK_ROUTE);
+    return sk_launch(k, ln_buf, K, W, K, bias, nullptr, out, ldo, R, N, K, flags, st, next_w, next_bytes, x, gamma, beta);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2160,37 +2054,17 @@ extern "C" mw_status mw_step_projection_h16(const void* d_x_h16, const float* d_
     MW_REQUIRE(!ln || !forced, "mw_step_projection_h16: path %d forces one projection kernel on x_h16: no LayerNorm", path);
     MW_REQUIRE(!ln || !d_resid, "mw_step_projection_h16: a LayerNorm projection takes no residual");
     MW_REQUIRE(!ln || (K % 128 == 0 && K <= 2048), "mw_step_projection_h16: LayerNorm over K=%d (a multiple of 128 up to 2048)", K);
-    const char* missing = nullptr;
-    switch (path) {
-        case MW_STEP_PATH_ROWS16_WT1: if (!sk_table_warps(K)) missing = "rows16"; break;
-        case MW_STEP_PATH_ROWS16_WT2: if (!sk_has_rows16_wt2(K)) missing = "two-tile rows16"; break;
-        case MW_STEP_PATH_KHALF_WT1: case MW_STEP_PATH_KHALF_WT2: if (!sk_has_khalf(K)) missing = "K-halved"; break;
-        case MW_STEP_PATH_LN_FUSED: if (!sk_has_ln_fused(K) || (flags & SK_FLAG_F32)) missing = "fused LayerNorm (16-bit output)"; break;
-        default: break;
-    }
-    if (missing) {
-        set_error("mw_step_projection_h16: no %s kernel for K=%d", missing, K);
-        return MW_ERR_UNSUPPORTED;
-    }
+    // LN_SEPARATE is the beam routing, whose LayerNorm is never fused
+    const SkKernel kernel_of_path[] = {SK_ROUTE, SK_ROUTE, SK_ROUTE, SK_ROUTE, SK_ROWS16_WT1, SK_ROWS16_WT2, SK_KHALF_WT1,
+                                       SK_KHALF_WT2, SK_GENERIC, SK_LN_FUSED, SK_ROUTE};
+    const SkKernel p = kernel_of_path[path];
+    const bool allow_dg = path == MW_STEP_PATH_GREEDY || path == MW_STEP_PATH_GREEDY_SOLO;
+    const bool solo = path == MW_STEP_PATH_GREEDY_SOLO || path == MW_STEP_PATH_BEAM_SOLO;
+    if (sk_choose(K, K, R, N, K, flags, p, allow_dg, solo, ln) == SK_NONE) return sk_missing("mw_step_projection_h16", p, K);
     MW_REQUIRE(d_x_h16 && d_w && d_out && (!ln || (d_x_f32 && d_gamma && d_beta)), "mw_step_projection_h16: null pointer");
     MW_REQUIRE((uintptr_t)d_x_h16 % 16 == 0 && (uintptr_t)d_w % 16 == 0 && (uintptr_t)d_x_f32 % 16 == 0,
                "mw_step_projection_h16: x and W must be 16-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
-    SkPath p = SK_ROUTE;
-    bool allow_dg = false, solo = false;
-    switch (path) {
-        case MW_STEP_PATH_GREEDY: allow_dg = true; break;
-        case MW_STEP_PATH_GREEDY_SOLO: allow_dg = true; solo = true; break;
-        case MW_STEP_PATH_BEAM_SOLO: solo = true; break;
-        case MW_STEP_PATH_ROWS16_WT1: p = SK_ROWS16_WT1; break;
-        case MW_STEP_PATH_ROWS16_WT2: p = SK_ROWS16_WT2; break;
-        case MW_STEP_PATH_KHALF_WT1: p = SK_KHALF_WT1; break;
-        case MW_STEP_PATH_KHALF_WT2: p = SK_KHALF_WT2; break;
-        case MW_STEP_PATH_GENERIC: p = SK_GENERIC; break;
-        case MW_STEP_PATH_LN_FUSED: p = SK_LN_FUSED; break;
-        case MW_STEP_PATH_LN_SEPARATE: p = SK_LN_SEPARATE; break;
-        default: break;
-    }
     if (ln)
         return skinny_gemm_ln(d_x_f32, d_gamma, d_beta, const_cast<void*>(d_x_h16), d_w, d_bias, d_out, N, R, N, K, flags, st,
                               allow_dg, nullptr, 0, solo, p);

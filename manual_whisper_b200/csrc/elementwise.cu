@@ -7,8 +7,6 @@ namespace mw {
 
 namespace {
 
-__device__ __forceinline__ float gelu_erf(float v) { return 0.5f * v * (1.0f + erff(v * 0.70710678118654752f)); }
-
 // one warp per row; d % 128 == 0, d <= 128 * MAXV.  MODE 0: LN -> h16; 1: GELU(LN) -> h16; 2: GELU(LN) -> f32;
 // 3: LN -> h16 AND f32 written back over x (post-LayerNorm encoders: the normalised row is both the next GEMM operand and
 // the residual stream)
@@ -28,43 +26,25 @@ layernorm_kernel(const float* x /* MODE 3 writes it back: no __restrict__ */, co
     for (int i = 0; i < MAXV; ++i)
         if (i < nv) {
             v[i] = xr[i * 32 + lane];
-            s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
+            s += sum4(v[i]);
         }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    const float mean = s / (float)d;
-    float q = 0.0f;
-#pragma unroll
-    for (int i = 0; i < MAXV; ++i)
-        if (i < nv) {
-            const float a = v[i].x - mean, b = v[i].y - mean, c = v[i].z - mean, e = v[i].w - mean;
-            q += (a * a + b * b) + (c * c + e * e);
-        }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
-    const float rstd = rsqrtf(q / (float)d + 1e-5f);
+    float mean, rstd;
+    ln_stats(s, v, nv, d, mean, rstd);
     const float4* g4 = reinterpret_cast<const float4*>(gamma);
     const float4* b4 = reinterpret_cast<const float4*>(beta);
     uint2* o2 = reinterpret_cast<uint2*>(out + (int64_t)row * d);
 #pragma unroll
     for (int i = 0; i < MAXV; ++i)
         if (i < nv) {
-            const float4 g = __ldg(g4 + i * 32 + lane), bb = __ldg(b4 + i * 32 + lane);
-            float y0 = (v[i].x - mean) * rstd * g.x + bb.x, y1 = (v[i].y - mean) * rstd * g.y + bb.y;
-            float y2 = (v[i].z - mean) * rstd * g.z + bb.z, y3 = (v[i].w - mean) * rstd * g.w + bb.w;
-            if (MODE == 1 || MODE == 2) { y0 = gelu_erf(y0); y1 = gelu_erf(y1); y2 = gelu_erf(y2); y3 = gelu_erf(y3); }
+            float4 y = ln_apply(v[i], mean, rstd, __ldg(g4 + i * 32 + lane), __ldg(b4 + i * 32 + lane));
+            if (MODE == 1 || MODE == 2) y = make_float4(gelu_erff(y.x), gelu_erff(y.y), gelu_erff(y.z), gelu_erff(y.w));
             if (MODE == 2) {
-                reinterpret_cast<float4*>(reinterpret_cast<float*>(out_v) + (int64_t)row * d)[i * 32 + lane] = make_float4(y0, y1, y2, y3);
+                reinterpret_cast<float4*>(reinterpret_cast<float*>(out_v) + (int64_t)row * d)[i * 32 + lane] = y;
                 continue;
             }
             if (MODE == 3)      // the row is held in registers: writing it back in place is safe
-                reinterpret_cast<float4*>(const_cast<float*>(x) + (int64_t)row * d)[i * 32 + lane] = make_float4(y0, y1, y2, y3);
-            mw_h2 h0 = f2h2(y0, y1);
-            mw_h2 h1 = f2h2(y2, y3);
-            uint2 u;
-            u.x = *reinterpret_cast<uint32_t*>(&h0);
-            u.y = *reinterpret_cast<uint32_t*>(&h1);
-            o2[i * 32 + lane] = u;
+                reinterpret_cast<float4*>(const_cast<float*>(x) + (int64_t)row * d)[i * 32 + lane] = y;
+            o2[i * 32 + lane] = pack_h16x4(y);
         }
 }
 

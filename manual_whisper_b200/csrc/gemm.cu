@@ -49,21 +49,6 @@ struct SmemLayout {
     static constexpr int TOTAL = BAR_OFF + (2 * STAGES + 4) * 8 + 16 + 1024;  // +1024: manual alignment slack
 };
 
-// Exact-erf GELU, 0.5 v (1 + erf(v / sqrt 2)), with erf from Abramowitz & Stegun 7.1.26 (|error| < 1.5e-7, far below the
-// bf16 rounding of the value that is stored): one MUFU.RCP, one MUFU.EX2 and seven FMAs instead of erff's ~25
-// instructions — the fc1 epilogue was issue-bound on erff.
-__device__ __forceinline__ float gelu_erf(float v) {
-    const float x = fabsf(v) * 0.70710678118654752f;
-    const float t = __fdividef(1.0f, fmaf(0.3275911f, x, 1.0f));
-    float p = fmaf(1.061405429f, t, -1.453152027f);
-    p = fmaf(p, t, 1.421413741f);
-    p = fmaf(p, t, -0.284496736f);
-    p = fmaf(p, t, 0.254829592f);
-    const float e = p * t * exp2f(-1.4426950408889634f * x * x);      // 1 - erf(x)
-    const float erf_abs = 1.0f - e;
-    return 0.5f * v * (1.0f + copysignf(erf_abs, v));
-}
-
 #ifndef MW_GEMM_MINBLOCKS
 #define MW_GEMM_MINBLOCKS 1
 #endif
@@ -213,7 +198,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
                     }
                     if (p.gelu) {
 #pragma unroll
-                        for (int j = 0; j < 32; ++j) v[j] = gelu_erf(v[j]);
+                        for (int j = 0; j < 32; ++j) v[j] = gelu_as7126(v[j]);
                     }
                     if (use_res) {
 #pragma unroll

@@ -1,4 +1,5 @@
-// Shared host-side plumbing of libmw_b200.so: error strings, launch counting, device guards.
+// Shared plumbing of libmw_b200.so: the 16-bit storage type, scalar device math several kernels share (GELU, LayerNorm rows),
+// error strings, launch counting, device guards.
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
@@ -46,6 +47,65 @@ __device__ __forceinline__ mw_h2 f2h2_bounded(float a, float b) { return __float
 #endif
 
 namespace mw {
+
+// ---- scalar device math shared by several kernels
+
+// GELU, 0.5 v (1 + erf(v / sqrt 2)), in two forms that differ in the last bits; each kernel keeps the form it was validated
+// with.  gelu_erff uses the library erff: the mma.sync decode projections, the LayerNorm + GELU kernels and wav2vec2.
+__device__ __forceinline__ float gelu_erff(float v) { return 0.5f * v * (1.0f + erff(v * 0.70710678118654752f)); }
+
+// gelu_as7126 takes erf from Abramowitz & Stegun 7.1.26 (|error| < 1.5e-7, far below the 16-bit rounding of the value that
+// is stored): one MUFU.RCP, one MUFU.EX2 and seven FMAs instead of erff's ~25 instructions - the tcgen05 GEMM's fc1 epilogue
+// was issue-bound on erff.  The two tcgen05 GEMMs (gemm.cu, decode_gemm.cu) use it.
+__device__ __forceinline__ float gelu_as7126(float v) {
+    const float x = fabsf(v) * 0.70710678118654752f;
+    const float t = __fdividef(1.0f, fmaf(0.3275911f, x, 1.0f));
+    float p = fmaf(1.061405429f, t, -1.453152027f);
+    p = fmaf(p, t, 1.421413741f);
+    p = fmaf(p, t, -0.284496736f);
+    p = fmaf(p, t, 0.254829592f);
+    const float e = p * t * exp2f(-1.4426950408889634f * x * x);      // 1 - erf(|x|)
+    return 0.5f * v * (1.0f + copysignf(1.0f - e, v));
+}
+
+__device__ __forceinline__ float warp_sum(float s) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    return s;
+}
+
+__device__ __forceinline__ float sum4(float4 v) { return (v.x + v.y) + (v.z + v.w); }
+
+// LayerNorm of a row of d = 128 nv floats held by one warp: lane l holds float4 i * 32 + l of the row in v[i], i < nv <= MAXV,
+// and s = the sum over i of sum4(v[i]), in order.  layernorm_kernel (elementwise.cu) and the fused projection
+// skinny_gemm_ln_kernel (decoder.cu) both normalise with these, so the 16-bit operands they produce are the same bits.
+template <int MAXV>
+__device__ __forceinline__ void ln_stats(float s, const float4 (&v)[MAXV], int nv, int d, float& mean, float& rstd) {
+    mean = warp_sum(s) / (float)d;
+    float q = 0.0f;
+#pragma unroll
+    for (int i = 0; i < MAXV; ++i)
+        if (i < nv) {
+            const float a = v[i].x - mean, b = v[i].y - mean, c = v[i].z - mean, e = v[i].w - mean;
+            q += (a * a + b * b) + (c * c + e * e);
+        }
+    rstd = rsqrtf(warp_sum(q) / (float)d + 1e-5f);
+}
+
+__device__ __forceinline__ float4 ln_apply(float4 v, float mean, float rstd, float4 g, float4 b) {
+    return make_float4((v.x - mean) * rstd * g.x + b.x, (v.y - mean) * rstd * g.y + b.y, (v.z - mean) * rstd * g.z + b.z,
+                       (v.w - mean) * rstd * g.w + b.w);
+}
+
+__device__ __forceinline__ uint2 pack_h16x4(float4 y) {
+    mw_h2 h0 = f2h2(y.x, y.y), h1 = f2h2(y.z, y.w);
+    uint2 u;
+    u.x = *reinterpret_cast<uint32_t*>(&h0);
+    u.y = *reinterpret_cast<uint32_t*>(&h1);
+    return u;
+}
+
+// ---- host-side plumbing
 
 void set_error(const char* fmt, ...);
 extern std::atomic<uint64_t> g_launches;

@@ -70,8 +70,6 @@ __host__ __device__ inline int conv_frames(int64_t n, int upto = 7) {
     return (int)t;
 }
 
-__device__ __forceinline__ float gelu_exact(float v) { return 0.5f * v * (1.0f + erff(v * 0.70710678118654752f)); }
-
 __global__ void w2v_frames_kernel(const int* __restrict__ lens, int n, int* __restrict__ frames) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) frames[i] = conv_frames(max(lens[i], 400));
@@ -135,8 +133,8 @@ w2v_conv0_kernel(const float* __restrict__ audio, int64_t n_audio, const int64_t
 #pragma unroll
         for (int p = 0; p < NP; ++p) {
             const int c = 2 * lane + 64 * p;
-            const float y0 = gelu_exact((v[p][0] - mean) * rstd * sg[c] + sbe[c]);
-            const float y1 = gelu_exact((v[p][1] - mean) * rstd * sg[c + 1] + sbe[c + 1]);
+            const float y0 = gelu_erff((v[p][0] - mean) * rstd * sg[c] + sbe[c]);
+            const float y1 = gelu_erff((v[p][1] - mean) * rstd * sg[c + 1] + sbe[c + 1]);
             *reinterpret_cast<mw_h2*>(o + c) = f2h2(y0, y1);
         }
     }
@@ -194,8 +192,8 @@ w2v_conv0_gn_kernel(const float* __restrict__ audio, int64_t n_audio, const int6
             if (MODE == 0) {
                 if (t < T0b) { ps[p][0] += a0; ps[p][1] += a1; pq[p][0] = fmaf(a0, a0, pq[p][0]); pq[p][1] = fmaf(a1, a1, pq[p][1]); }
             } else {
-                const float y0 = t < T0b ? gelu_exact(fmaf(a0, red[0][c], red[0][C + c])) : 0.0f;
-                const float y1 = t < T0b ? gelu_exact(fmaf(a1, red[0][c + 1], red[0][C + c + 1])) : 0.0f;
+                const float y0 = t < T0b ? gelu_erff(fmaf(a0, red[0][c], red[0][C + c])) : 0.0f;
+                const float y1 = t < T0b ? gelu_erff(fmaf(a1, red[0][c + 1], red[0][C + c + 1])) : 0.0f;
                 *reinterpret_cast<mw_h2*>(o + c) = f2h2(y0, y1);
             }
         }
@@ -262,7 +260,7 @@ w2v_pos_add_kernel(const float* __restrict__ tmp, const float* __restrict__ bias
     const int64_t r = i / d;
     const int c = (int)(i - r * d), g = c / gw, ci = c - g * gw;
     const int G = d / gw;
-    x[i] += gelu_exact(tmp[r * (int64_t)(G * 64) + g * 64 + ci] + bias[c]);
+    x[i] += gelu_erff(tmp[r * (int64_t)(G * 64) + g * 64 + ci] + bias[c]);
 }
 
 // logits f32 [n*T, ldl] -> log_softmax over the first V columns, written to the caller's [frames_c, V] block of window c

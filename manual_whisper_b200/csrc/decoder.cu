@@ -14,6 +14,7 @@
 #include "model.cuh"
 #include "gemm.cuh"
 #include "kernels.cuh"
+#include "ptx_sm100.cuh"
 
 #include <algorithm>
 #include <stdlib.h>
@@ -110,10 +111,12 @@ __device__ __forceinline__ void mma_h16_16816(float (&c)[4], uint32_t a0, uint32
         : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
+// A weight load: a weight byte is read once per step, so its line is marked evict_first in L2.  `volatile` keeps the loads
+// in program order ahead of the MMAs, so a kernel's whole weight slice is in flight before the first MMA waits.
 __device__ __forceinline__ uint4 ldg_stream(const void* p) {
     uint4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;"
+                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p), "l"(ptx::l2_policy_evict_first()));
     return r;
 }
 
@@ -121,11 +124,17 @@ __device__ __forceinline__ uint4 ldg_stream(const void* p) {
 // per launch with nothing else in flight).  Every projection kernel therefore asks L2 for the NEXT projection's weight
 // matrix once its own weights have arrived (`pf`, `pf_lines` 128-byte lines, spread over the grid's threads), so the next
 // kernel's stream starts from L2; the cross-attention kernel does the same for its output projection.
+// With several batches in flight, the other batches stream cross-attention K/V and self-attention K/V through L2 between
+// the prefetch and the load that consumes it.  Those streams are loaded evict_first and the prefetch marks its lines
+// evict_last, so L2 gives up the streamed lines first and the prefetched weights are still there when they are read.
+// The consuming load (ldg_stream) is evict_first, and a hinted access re-marks a resident line (the PTX ISA's
+// evict_unchanged priority exists to opt out of that), so a weight line is demoted once it has been read and evict_last
+// lines do not pile up: at any time they are at most the next matrix of each batch in flight.
 __device__ __forceinline__ void l2_prefetch_slice(const char* pf, int pf_lines) {
     if (!pf) return;
     const int nthr = gridDim.x * gridDim.y * blockDim.x;
     for (int i = (blockIdx.y * gridDim.x + blockIdx.x) * blockDim.x + threadIdx.x; i < pf_lines; i += nthr)
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(pf + (int64_t)i * 128));
+        ptx::prefetch_l2_evict_last(pf + (int64_t)i * 128);
 }
 
 // The weight fragments of WT tiles (rows n0 + 16 wt + g and + 8, clamped to N - 1) x KB blocks from column k0 (q * 8 included)
@@ -193,8 +202,9 @@ __device__ __forceinline__ void sk_output(float (*red)[32][LD], int rl, int nl, 
     }
 }
 
-// Any K % 32 == 0: grid (ceil(N/16), ceil(R/32)), 256 threads; warp w owns K blocks w, w+8, ...
-__global__ void __launch_bounds__(256)
+// Any K % 32 == 0: grid (ceil(N/16), ceil(R/32)), 256 threads; warp w owns K blocks w, w+8, ...  At most 64 registers, so
+// 4 CTAs fit an SM (the cache policy of the weight loads would otherwise take it to 70 and 3 CTAs).
+__global__ void __launch_bounds__(256, 4)
 skinny_gemm_kernel(const mw_h* __restrict__ X, int ldx, const mw_h* __restrict__ W, int ldw,
                    const float* __restrict__ bias, const float* resid, void* out, int ldo, int R, int N, int K,
                    int flags) {
@@ -574,6 +584,10 @@ decode_attn_kernel(const mw_h* __restrict__ q, int ldq,
         __syncthreads();
     }
     const int* idx = (SELF && idx_table) ? idx_table + (int64_t)r * ctx : nullptr;
+    // The self K/V cache is read once per step and is larger than L2 with several batches in flight, so its lines go first
+    // (ld.global.cs: evict-first in L1 and L2).  It is a coherent load because this kernel appends to the cache; the
+    // batched prefill reads activations and keeps the default policy.
+    auto kv_load = [](const mw_h* p) { return SELF ? __ldcs(reinterpret_cast<const uint4*>(p)) : *reinterpret_cast<const uint4*>(p); };
     float qf[8];
     {
         const uint4 u = *reinterpret_cast<const uint4*>(q + (int64_t)r * ldq + h * 64 + lg * 8);
@@ -591,7 +605,7 @@ decode_attn_kernel(const mw_h* __restrict__ q, int ldq,
             const int key = key0 + 16 * u;
             if (key < n_keys) {
                 const int seq = idx ? ((key == n_keys - 1) ? r : idx[key]) : (SELF ? r : seq0);
-                kv[u] = *reinterpret_cast<const uint4*>(kbase + ((int64_t)seq * keys_per_seq + key) * key_stride + h * 64 + lg * 8);
+                kv[u] = kv_load(kbase + ((int64_t)seq * keys_per_seq + key) * key_stride + h * 64 + lg * 8);
             }
         }
 #pragma unroll
@@ -641,7 +655,7 @@ decode_attn_kernel(const mw_h* __restrict__ q, int ldq,
             const int key = key0 + 16 * u;
             if (key < n_keys) {
                 const int seq = idx ? ((key == n_keys - 1) ? r : idx[key]) : (SELF ? r : seq0);
-                vv[u] = *reinterpret_cast<const uint4*>(vbase + ((int64_t)seq * keys_per_seq + key) * key_stride + h * 64 + lg * 8);
+                vv[u] = kv_load(vbase + ((int64_t)seq * keys_per_seq + key) * key_stride + h * 64 + lg * 8);
             }
         }
 #pragma unroll
@@ -696,6 +710,7 @@ cross_attn_stream_kernel(const mw_h* __restrict__ q, int ldq, const mw_h* __rest
     const int lg = lane & 7, kq = lane >> 3;
     const mw_h* kp = kbase + (int64_t)r * n_keys * key_stride + h * 64 + lg * 8;
     const mw_h* vp = vbase + (int64_t)r * n_keys * key_stride + h * 64 + lg * 8;
+    const uint64_t pol = ptx::l2_policy_evict_first();     // K/V are read once per step: let them go before the prefetched weights
     float qf[8];
     {
         const uint4 u = *reinterpret_cast<const uint4*>(q + (int64_t)r * ldq + h * 64 + lg * 8);
@@ -713,8 +728,8 @@ cross_attn_stream_kernel(const mw_h* __restrict__ q, int ldq, const mw_h* __rest
         for (int u = 0; u < UNR; ++u) {
             const int key = key0 + 16 * u;
             if (key < key_hi) {
-                kv[u] = *reinterpret_cast<const uint4*>(kp + (int64_t)key * key_stride);
-                vv[u] = *reinterpret_cast<const uint4*>(vp + (int64_t)key * key_stride);
+                kv[u] = ptx::ldg_nc_hint(kp + (int64_t)key * key_stride, pol);
+                vv[u] = ptx::ldg_nc_hint(vp + (int64_t)key * key_stride, pol);
             }
         }
         float sv[UNR];
@@ -802,6 +817,7 @@ cross_attn_grouped_kernel(const mw_h* __restrict__ q, int ldq, const mw_h* __res
     }
     const mw_h* kb = kbase + (int64_t)b * n_keys * key_stride + h * 64 + lg * 8;
     const mw_h* vb = vbase + (int64_t)b * n_keys * key_stride + h * 64 + lg * 8;
+    const uint64_t pol = ptx::l2_policy_evict_first();     // K and V are read once per step, as in cross_attn_stream_kernel
     // Scores: every lane forms 8-dim partial dots for all G queries; a 3-round reduce-scatter over the 8 lanes of a key
     // (4 + 2 + 1 shuffles instead of 3 per query) leaves lane lg with the complete score of query lg.
     const bool b2 = lg & 4, b1 = lg & 2, b0 = lg & 1;
@@ -812,7 +828,7 @@ cross_attn_grouped_kernel(const mw_h* __restrict__ q, int ldq, const mw_h* __res
 #pragma unroll
         for (int u = 0; u < UNR; ++u) {
             const int key = key0 + 16 * u;
-            if (key < n_keys) kv[u] = *reinterpret_cast<const uint4*>(kb + (int64_t)key * key_stride);
+            if (key < n_keys) kv[u] = ptx::ldg_nc_hint(kb + (int64_t)key * key_stride, pol);
         }
 #pragma unroll
         for (int u = 0; u < UNR; ++u) {
@@ -880,7 +896,7 @@ cross_attn_grouped_kernel(const mw_h* __restrict__ q, int ldq, const mw_h* __res
 #pragma unroll
         for (int u = 0; u < UNR; ++u) {
             const int key = key0 + 16 * u;
-            if (key < n_keys) vv[u] = *reinterpret_cast<const uint4*>(vb + (int64_t)key * key_stride);
+            if (key < n_keys) vv[u] = ptx::ldg_nc_hint(vb + (int64_t)key * key_stride, pol);
         }
 #pragma unroll
         for (int u = 0; u < UNR; ++u) {

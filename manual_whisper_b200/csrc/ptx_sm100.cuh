@@ -31,6 +31,30 @@ __device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
     return d;
 }
 
+// ------------------------------------------------------------------ L2 eviction priority
+// A cache policy (createpolicy) carried by a load as `.L2::cache_hint` sets the L2 eviction priority of the lines it touches.
+// The PTX ISA's priority list includes evict_unchanged ("do not change eviction priority order as part of this access"),
+// which implies that an access with any other priority re-marks a line that is already resident.  Hints may be ignored by
+// the hardware; they never change what a load returns.  The policy is a pure value (no `volatile`): ptxas folds it into
+// the load's uniform memory descriptor.
+__device__ __forceinline__ uint64_t l2_policy_evict_first() {
+    uint64_t p;
+    asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
+    return p;
+}
+// 16 read-only bytes, not allocated in L1, with an L2 cache policy.  Not `volatile`: the data must not change during the
+// kernel (ld.global.nc), so the compiler may schedule the load freely.
+__device__ __forceinline__ uint4 ldg_nc_hint(const void* p, uint64_t pol) {
+    uint4 r;
+    asm("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;"
+        : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p), "l"(pol));
+    return r;
+}
+// the 128-byte line holding p into L2, marked evict_last
+__device__ __forceinline__ void prefetch_l2_evict_last(const void* p) {
+    asm volatile("prefetch.global.L2::evict_last [%0];" ::"l"(p));
+}
+
 // ------------------------------------------------------------------ mbarrier
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
